@@ -3,6 +3,7 @@
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--config c1|c2|c2h|c3|c4|c5] [--impl ours|reference]
                     [--engine auto|simt_fp32|tc_3x|tc_3x_w1 (reduced precision, labelled so)] [--graph 0|1] [--device cpu|cuda (reference arm)]
+                    [--dump-outputs DIR]
 
 One "step" = one pass of the hot path over one synthetic ray batch of a BASELINE config, through the public API
 (`Graph.render_image_at_specific_rays` + the loss module's `compute_loss` + `backward()`), gradients zeroed each step:
@@ -22,9 +23,14 @@ CUDA events on the launching stream, with an L2 flush (256 MiB memset) between s
 a synchronize after each step; ms_per_step = mean of the K intervals, MAX over ranks.  `--sync-each-step 0` enqueues the K
 steps back to back instead.  Clocks / throttle reasons are sampled with nvidia-smi during the timed region.  Prints ONE JSON line (rank 0).
 
-`--impl reference` times the UNMODIFIED reference (oracle/_ref, made by oracle/build_ref.py) on the host cores
-(`--device cuda`: on the GPU, the torch/cuBLAS path SURVEY 8d calls "the kernel to beat"); without oracle/_ref it
-falls back to the oracle port.  The N = 1 line of our arm carries both as `cpu_baseline` and `torch_gpu_baseline`.
+`--impl reference` times the torch restatement of the reference's hot path (oracle/sparf_oracle.py, pinned to the
+reference by tests/golden; config c2) on the host cores (`--device cuda`: on the GPU, the torch/cuBLAS path SURVEY 8d
+calls "the kernel to beat").  The N = 1 line of our arm carries both as `cpu_baseline` and `torch_gpu_baseline`.
+
+`--dump-outputs DIR` writes what the last timed step of our arm computed, as DIR/<name>.npy: the loss, every parameter
+gradient (`grad.graph.*`, `grad.pose.*`) and the tensors the render call returned (`render.*`), rank 0.  The inputs
+(scene, weights, ray draws, sampling noise) are seeded, so two builds run with the same arguments can be compared
+array by array.
 """
 from __future__ import annotations
 
@@ -148,17 +154,8 @@ class _TrainData:
         return self.n
 
 
-def reference_modules():
-    """The unmodified reference's classes (oracle/ref_loader.py), or None when neither /root/reference nor oracle/_ref exists."""
-    from oracle import ref_loader
-    if not ref_loader.ref_root():
-        return None
-    return ref_loader.load("trainer")
-
-
-def build_problem(cfg_name, impl, device, seed=0, stratified=True):
-    """Model + data + loss module of one BASELINE config, for our path (impl='ours') or the reference's own classes
-    (impl='reference': same constructor calls -- that is the drop-in contract).  Returns a namespace with `.step(ray_idx)`."""
+def build_problem(cfg_name, device, seed=0, stratified=True):
+    """Model + data + loss module of one BASELINE config on our path.  Returns a namespace with `.forward_backward(ray_idx)`."""
     import common
     cfg = CONFIGS[cfg_name]
     B, H, W = cfg["B"], cfg["H"], cfg["W"]
@@ -177,14 +174,9 @@ def build_problem(cfg_name, impl, device, seed=0, stratified=True):
         data[k] = data[k].to(device)
     sd = common.det_weights(opt, seed, progress=cfg["progress"])
     sd_fine = common.det_weights(opt, seed + 77, progress=cfg["progress"]) if cfg["fine"] else None
-    if impl == "ours":
-        from sparf_b200.losses import define_loss
-        from sparf_b200.poses_models import FirstTwoColunmnsPoseParameters
-        from sparf_b200.renderer import Graph
-    else:
-        ref = reference_modules()
-        Graph, FirstTwoColunmnsPoseParameters = ref.renderer.Graph, ref.two_columns.FirstTwoColunmnsPoseParameters
-        define_loss = ref.loss_factory.define_loss
+    from sparf_b200.losses import define_loss
+    from sparf_b200.poses_models import FirstTwoColunmnsPoseParameters
+    from sparf_b200.renderer import Graph
     pose_net = None
     if cfg["poses"]:
         init = common.perturb_poses(data.pose.cpu(), seed, sigma=0.02).to(device)
@@ -202,10 +194,8 @@ def build_problem(cfg_name, impl, device, seed=0, stratified=True):
         net.nerf_fine.load_state_dict(sd_fine)
     net.to(device).train()
     flow = common.FakeFlowNet(B, H, W) if "corres" in cfg["loss_type"] else None
-    if impl == "ours":   # sync-free fixed-shape mode of the SPARF losses (SURVEY 8f.2): the step is one CUDA graph
-        loss_module = define_loss(opt.loss_type, opt, net, _TrainData(data, B), device, flow_net=flow, device_side=True)
-    else:
-        loss_module = define_loss(opt.loss_type, opt, net, _TrainData(data, B), device, flow_net=flow)
+    # sync-free fixed-shape mode of the SPARF losses (SURVEY 8f.2): the step is one CUDA graph
+    loss_module = define_loss(opt.loss_type, opt, net, _TrainData(data, B), device, flow_net=flow, device_side=True)
     modules = [net] + ([pose_net] if pose_net is not None else [])
     pr = argparse.Namespace(cfg=cfg, opt=opt, data=data, net=net, pose_net=pose_net, loss_module=loss_module,
                             modules=modules, iteration=10)
@@ -221,7 +211,7 @@ def build_problem(cfg_name, impl, device, seed=0, stratified=True):
         loss.backward()
         if needs_poses:     # do not keep the step's autograd graph alive into the next step (or a graph capture)
             data.pop("poses_w2c", None)
-        return loss.detach()
+        return loss.detach(), {k: v.detach() for k, v in out.items() if torch.is_tensor(v)}
 
     pr.forward_backward = forward_backward
     return pr
@@ -262,7 +252,7 @@ def run_ours(args):
     cfg = CONFIGS[args.config]
     strong = cfg["scaling"] == "strong"
     # weak scaling: every rank its own scene-independent batch (seed = rank); strong: one global batch, sharded
-    pr = build_problem(args.config, "ours", dev, seed=0 if strong else rank)
+    pr = build_problem(args.config, dev, seed=0 if strong else rank)
     pr.net.device_side_rng = True
     pr.loss_module.check_finite = False      # no host synchronisation inside the step (see sparf_b200/losses.py)
     if world > 1:   # identical replicas of the MLPs / poses on every rank
@@ -289,18 +279,18 @@ def run_ours(args):
     loss_host = torch.zeros((), pin_memory=True)
     scale = (n_view / n_view_global) if (strong and world > 1) else 1.0   # local mean -> share of the global mean
 
-    def local_step(ray_idx_dev):   # everything of a step except the cross-rank exchange
+    def local_step(ray_idx_dev):   # everything of a step except the cross-rank exchange -> (loss, render outputs)
         flat.zero_()
-        loss = pr.forward_backward(ray_idx_dev)
+        out = pr.forward_backward(ray_idx_dev)
         if scale != 1.0:
             flat.mul_(scale)
-        return loss
+        return out
 
     def step(ray_idx_dev):
-        loss = local_step(ray_idx_dev)
+        out = local_step(ray_idx_dev)
         if world > 1:
             dist.all_reduce(flat)  # one NCCL all-reduce of [d theta | d xi] per step (SURVEY 8e)
-        return loss
+        return out
 
     graphed, ar_in_graph, launches_per_graph = None, False, None
     evals_per_step = None
@@ -328,10 +318,10 @@ def run_ours(args):
             torch.cuda.synchronize()
 
     def graph_step(ray_idx_src):
-        loss = graphed(ray_idx_src)
+        out = graphed(ray_idx_src)
         if world > 1 and not ar_in_graph:
             dist.all_reduce(flat)
-        return loss
+        return out
 
     def timed(n_warm, n_steps, e2e, use_graph=False):
         # every step is bracketed by its own pair of CUDA events on the launching stream with the L2 flush outside the
@@ -342,7 +332,7 @@ def run_ours(args):
         if world > 1:
             dist.barrier()
         torch.cuda.synchronize()
-        events = []
+        events, render = [], None
         for i in range(n_warm + n_steps):
             src = idx_host[(n_total if e2e else 0) + i]
             if not e2e:
@@ -352,7 +342,7 @@ def run_ours(args):
             e0.record()
             if e2e:  # host buffers in, host scalar out, inside the timed region
                 ray_idx_dev = src if use_graph else src.to(dev, non_blocking=True)
-            loss = graph_step(ray_idx_dev) if use_graph else step(ray_idx_dev)
+            loss, render = graph_step(ray_idx_dev) if use_graph else step(ray_idx_dev)
             if e2e:
                 loss_host.copy_(loss.detach(), non_blocking=True)
             e1.record()
@@ -366,7 +356,7 @@ def run_ours(args):
         t = torch.tensor([sum(times)], device=dev, dtype=torch.float64)
         if world > 1:
             dist.all_reduce(t, op=dist.ReduceOp.MAX)
-        return float(t.item()), times
+        return float(t.item()), times, render
 
     rays_local = cfg["B"] * n_view
     rays_per_step = cfg["B"] * n_view_global if strong else rays_local * world
@@ -378,16 +368,24 @@ def run_ours(args):
     launches0 = L.sparf_launch_count()
     ops.PROFILE.clear()
     ops.PROFILE_ON[0] = True
-    total_ms, times = timed(0, args.steps, False)
+    total_ms, times, _ = timed(0, args.steps, False)
     ops.PROFILE_ON[0] = False
     launches = L.sparf_launch_count() - launches0
     mlp_ms = ops.profile_total_ms()   # MLP kernel groups timed with CUDA events in the eager pass (same kernels)
     eager_ms_per_step = total_ms / args.steps
     if graphed is not None:           # the reported step: one CUDA-graph replay per step
         timed(args.warmup, 0, False, use_graph=True)
-        total_ms, times = timed(0, args.steps, False, use_graph=True)
+        total_ms, times, _ = timed(0, args.steps, False, use_graph=True)
         launches = launches_per_graph * args.steps
-    e2e_ms, _ = timed(args.warmup, args.steps, True, use_graph=graphed is not None)
+    e2e_ms, _, render = timed(args.warmup, args.steps, True, use_graph=graphed is not None)
+    if args.dump_outputs and rank == 0:    # before the all-reduce timing below, which keeps summing into the gradients
+        arrays = {"loss": loss_host}
+        for prefix, m in (("grad.graph", pr.net), ("grad.pose", pr.pose_net)):
+            for name, p in (m.named_parameters() if m is not None else ()):
+                if p.grad is not None:
+                    arrays["%s.%s" % (prefix, name)] = p.grad
+        arrays.update(("render." + k, v) for k, v in render.items() if v.is_floating_point())
+        dump_outputs(args.dump_outputs, arrays)
     # cost of the collective alone (rank 0's view): the all-reduce of the flat buffer, timed back to back
     ar_us = None
     if world > 1:
@@ -444,7 +442,10 @@ def run_ours(args):
             tgb = torch_gpu_baseline(args.config, dev)
         except Exception as e:
             tgb = dict(unavailable="%s: %s" % (type(e).__name__, str(e)[:160]))
-        cpu = cpu_baseline(args.config, budget_s=25.0)
+        try:
+            cpu = cpu_baseline(args.config, budget_s=25.0)
+        except RuntimeError as e:   # a config the oracle port does not cover
+            cpu = dict(unavailable="%s: %s" % (type(e).__name__, str(e)[:160]))
     line = dict(metric=METRIC, value=value, unit="rays/s", n_gpus=world, steps=args.steps,
                 warmup=args.warmup, ms_per_step=ms_per_step, higher_is_better=True, scaling=cfg["scaling"], vs_baseline=None,
                 dtype=ENGINE_DTYPE.get(args.engine, "fp32 (CUDA cores)"), data="synthetic",
@@ -466,6 +467,22 @@ def run_ours(args):
     print(json.dumps(line), flush=True)
     if world > 1:
         shutdown_distributed(dist)
+
+
+def dump_outputs(dirname, arrays, limit_bytes=64 << 20):
+    """Write every tensor of `arrays` as dirname/<name>.npy in float32 (float64 stays float64).  If they come to more than
+    `limit_bytes` together, each array above an equal share of the limit is cut to a fixed, seeded sample of its
+    flattened values (the same positions on every run of the same configuration)."""
+    os.makedirs(dirname, exist_ok=True)
+    host = {k: v.detach().cpu().numpy() for k, v in arrays.items()}
+    host = {k: v if v.dtype == np.float64 else v.astype(np.float32) for k, v in host.items()}
+    share = limit_bytes // max(len(host), 1)
+    big = sum(v.nbytes for v in host.values()) > limit_bytes
+    for k, v in host.items():
+        if big and v.nbytes > share:
+            keep = np.sort(np.random.default_rng(0).choice(v.size, share // v.itemsize, replace=False))
+            v = v.reshape(-1)[keep]
+        np.save(os.path.join(dirname, k + ".npy"), v)
 
 
 def shutdown_distributed(dist, grace_s=15.0):
@@ -495,26 +512,14 @@ TRAFFIC_SOURCE = {"tc_3x": "profiles/r02_ncu_chain.md (ncu --set full of tc_mlp_
 
 # ------------------------------------------------------------------------------------------------ reference arms
 def reference_step_fn(cfg_name, device):
-    """One step of the hot path through the UNMODIFIED reference (oracle/_ref) on `device`; falls back to the oracle
-    port (config c2 only) when the reference copy is absent.  Returns (step, kind)."""
+    """One step of the hot path through the oracle port of the reference (oracle/sparf_oracle.py, config c2 only) on
+    `device`.  Returns (step, kind)."""
     cfg = CONFIGS[cfg_name]
     HW = cfg["H"] * cfg["W"]
     n_view = cfg["rand_rays"] // cfg["B"]
     g = torch.Generator().manual_seed(0)
-    if reference_modules() is not None:
-        import contextlib
-        with contextlib.redirect_stdout(sys.stderr):     # the reference prints progress ("Computing flows ...")
-            pr = build_problem(cfg_name, "reference", device, seed=0)
-        params = [p for m in pr.modules for p in m.parameters()]
-
-        def step():
-            for p in params:
-                p.grad = None
-            return pr.forward_backward(torch.randperm(HW, generator=g)[:n_view].to(device))
-
-        return step, "reference"
     if cfg_name != "c2":
-        raise RuntimeError("oracle/_ref is absent and the oracle port only covers config c2")
+        raise RuntimeError("the oracle port only covers config c2")
     import common
     from oracle import sparf_oracle as O
     opt = common.make_opt(S=cfg["S"], fine=False, stratified=True)
@@ -587,8 +592,7 @@ def cpu_baseline(cfg_name, budget_s=25.0):
     return dict(value=n_rays / dt, unit="rays/s", cores=used, host_cores=cores, kind=kind,
                 sample="%d full steps of config %s (%d rays) through %s on the host cores, torch CPU fp32, best thread "
                        "count of %s = %d, %.2f s/step"
-                       % (n, cfg_name, n_rays, "the unmodified reference (oracle/_ref)" if kind == "reference"
-                          else "oracle/sparf_oracle.py", tried, used, dt))
+                       % (n, cfg_name, n_rays, "oracle/sparf_oracle.py", tried, used, dt))
 
 
 def torch_gpu_baseline(cfg_name, dev, steps=10, warmup=3):
@@ -631,7 +635,7 @@ def run_reference(args):
     world = int(os.environ.get("WORLD_SIZE", "1"))
     if args.device == "cuda":
         dev = torch.device("cuda", int(os.environ.get("LOCAL_RANK", "0")))
-        tgb = torch_gpu_baseline(args.config, dev, steps=max(args.steps, 3), warmup=max(args.warmup, 1))
+        tgb = torch_gpu_baseline(args.config, dev, steps=args.steps, warmup=max(args.warmup, 1))
         v, kind, cores, dt = tgb["fp32"], tgb["kind"], 0, tgb["fp32_ms_per_step"] * 1e-3
         sample = "each step = the full batch on the GPU (eager PyTorch fp32, TF32 off); tf32: %.0f rays/s" % tgb["tf32"]
     else:
@@ -650,9 +654,7 @@ def run_reference(args):
                 dtype="fp32 (torch CPU)" if args.device != "cuda" else "fp32 (torch CUDA, TF32 off)", data="synthetic",
                 config=dict(workload=cfg["desc"], name=args.config, rays_per_gpu=n_rays, global_rays=n_rays,
                             samples_per_ray=cfg["S"], fine_samples_per_ray=(cfg["S"] + cfg["S_fine"]) if cfg["fine"] else 0,
-                            note=("the unmodified reference (git-ignored copy oracle/_ref made by oracle/build_ref.py), its own "
-                                  "Graph + loss modules" if kind == "reference" else
-                                  "oracle/_ref absent: timed on the torch restatement oracle/sparf_oracle.py, pinned to the reference by tests/golden")),
+                            note="timed on the torch restatement oracle/sparf_oracle.py, pinned to the reference by tests/golden"),
                 cpu_baseline=dict(value=v, unit="rays/s", cores=cores, kind=kind, sample=sample),
                 e2e=dict(value=v, unit="rays/s", h2d_bytes_per_step=0, d2h_bytes_per_step=0))
     print(json.dumps(line))
@@ -673,13 +675,15 @@ def main():
     ap.add_argument("--graph", type=int, default=1, help="1: replay the step as one CUDA graph (default), 0: eager")
     ap.add_argument("--allreduce-in-graph", type=int, default=1)
     ap.add_argument("--no-baselines", action="store_true", help="skip the cpu_baseline / torch_gpu_baseline legs")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the loss, gradients and render outputs of the last timed step as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
     if args.impl == "reference":
-        # bounded CPU sample (~1.2 s per c2 step on the best thread count): same step count as our arm up to 20
-        cap = 20 if args.config == "c2" else 5
-        if args.device == "cpu" and args.steps > cap:
-            args.steps = cap
+        if args.dump_outputs:
+            ap.error("--dump-outputs applies to --impl ours")
         run_reference(args)
     else:
         run_ours(args)

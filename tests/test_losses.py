@@ -147,41 +147,6 @@ def test_full_sparf_step_vs_reference(name, engine):
                    gtol=0.5 if inv else 6e-2, gnorm="l2" if inv else "max")
 
 
-@pytest.mark.gpu
-@pytest.mark.parametrize("name", ["c7_sparf_losses", "c9_colmap_depth"])
-def test_reference_trainer_graph_and_losses_on_our_renderer(name):
-    """THE DROP-IN PROOF.  The reference's OWN `joint_pose_nerf_trainer.Graph` subclass (:710-749), its own pose model
-    and its own `loss_factory.define_loss` modules run UNCHANGED with `source.models.renderer` resolved to
-    `sparf_b200.renderer` (oracle/ref_loader.py shadow_renderer=True): every render they trigger goes through the CUDA
-    kernels, and the losses / gradients must match the goldens the unmodified reference produced on its own renderer."""
-    from oracle import ref_loader
-    if not ref_loader.ref_root():
-        pytest.skip("oracle/_ref not built (python oracle/build_ref.py in the build container)")
-    import sparf_b200
-    import sparf_b200.renderer as our_renderer
-
-    sparf_b200.set_engine("auto")
-    ref = ref_loader.load("trainer", shadow_renderer=True)
-    try:
-        assert issubclass(ref.joint.Graph, our_renderer.Graph) and ref.joint.Graph is not our_renderer.Graph
-        dev = torch.device("cuda")
-        gold, c, opt, data, ray_idx, sd, sd_fine, init_w2c = _loss_case_setup(name, dev)
-        pose_net = ref.two_columns.FirstTwoColunmnsPoseParameters(opt, nbr_poses=c["B"], initial_poses_w2c=init_w2c, device=dev)
-        net = ref.joint.Graph(opt, dev, pose_net)
-        net.nerf.load_state_dict(sd)
-        if c["fine"]:
-            net.nerf_fine.load_state_dict(sd_fine)
-        net.to(dev).train()
-        flow = common.FakeFlowNet(c["B"], c["H"], c["W"])
-        np.random.seed(c["seed"])
-        loss_module = ref.loss_factory.define_loss(opt.loss_type, opt, net, _TrainData(data, c["B"]), dev, flow_net=flow)
-        assert type(loss_module).__module__.startswith("source.training.core")
-        _run_and_check(name, "reference trainer Graph + reference losses over sparf_b200 (auto engine)", gold, c, opt, data,
-                       ray_idx, net, loss_module, pose_net.pose_embedding, gtol=6e-2)
-    finally:
-        ref_loader._purge()
-
-
 def _sparf_problem(dev, stratified):
     import sparf_b200
     from sparf_b200.poses_models import FirstTwoColunmnsPoseParameters

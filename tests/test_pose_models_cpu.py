@@ -1,8 +1,8 @@
-"""Pose-parameter modules vs the reference's own modules, imported from /root/reference when it is mounted (the build
-container); on the GPU box the reference is absent and the comparison is skipped (the golden-backed tests remain)."""
+"""Pose-parameter modules vs the reference's own modules.  What the reference's QuaternionsPoseParameters computed on
+the inputs below is stored in golden/reference_modules.npz (tests/golden/make_module_golden.py regenerates it)."""
 import os
-import sys
 
+import numpy as np
 import pytest
 import torch
 
@@ -10,7 +10,8 @@ import common
 from sparf_b200.poses_models import QuaternionsPoseParameters
 from sparf_b200.utils.edict import edict
 
-HAVE_REF = os.path.isdir("/root/reference/source")
+GOLDEN = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "reference_modules.npz")
+REFERENCE_CASES = [(False, False, True, True), (True, True, True, True), (True, False, False, True), (False, True, True, False)]
 
 
 def _opt(c2w, rel, rot=True, trans=True):
@@ -37,24 +38,29 @@ def test_quaternion_pose_model_round_trip_and_gradients(c2w, rel):
     assert m.rot_embedding.grad.abs().sum() > 0 and m.trans_embedding.grad.abs().sum() > 0
 
 
-@pytest.mark.skipif(not HAVE_REF, reason="reference checkout not mounted")
-@pytest.mark.parametrize("c2w,rel,rot,trans", [(False, False, True, True), (True, True, True, True), (True, False, False, True),
-                                               (False, True, True, False)])
-def test_quaternion_pose_model_matches_reference_module(c2w, rel, rot, trans):
-    here = os.path.dirname(os.path.abspath(__file__))
-    for p in (os.path.join(here, "golden", "_shims"), "/root/reference"):
-        if p not in sys.path:
-            sys.path.insert(0, p)
-    from source.models.poses_models.quaternion import QuaternionsPoseParameters as Ref
+def quaternion_pose_run(cls, c2w, rel, rot, trans):
+    """Build a pose model of class `cls`, move it off its initial value, and return what it computes."""
     w2c = _poses(5)
-    opt = _opt(c2w, rel, rot, trans)
-    ours, ref = QuaternionsPoseParameters(opt, 4, w2c, torch.device("cpu")), Ref(opt, 4, w2c, torch.device("cpu"))
-    assert torch.allclose(torch.as_tensor(ours.rot_embedding), torch.as_tensor(ref.rot_embedding), atol=1e-6)
-    with torch.no_grad():       # move both off the initial value the same way
-        for m in (ours, ref):
-            if rot:
-                m.rot_embedding += 0.05 * torch.arange(m.rot_embedding.numel()).view_as(m.rot_embedding).float().cos()
-            if trans:
-                m.trans_embedding += 0.1
-    assert torch.allclose(ours.get_w2c_poses(), ref.get_w2c_poses(), atol=1e-6)
-    assert torch.allclose(ours.get_c2w_poses(), ref.get_c2w_poses(), atol=1e-6)
+    m = cls(_opt(c2w, rel, rot, trans), 4, w2c, torch.device("cpu"))
+    out = dict(rot_embedding=torch.as_tensor(m.rot_embedding).detach().clone())
+    with torch.no_grad():       # move off the initial value the same way for every implementation
+        if rot:
+            m.rot_embedding += 0.05 * torch.arange(m.rot_embedding.numel()).view_as(m.rot_embedding).float().cos()
+        if trans:
+            m.trans_embedding += 0.1
+    out["w2c"] = m.get_w2c_poses().detach()
+    out["c2w"] = m.get_c2w_poses().detach()
+    return out
+
+
+def pose_golden_key(c2w, rel, rot, trans, name):
+    return "quaternion_%d%d%d%d_%s" % (c2w, rel, rot, trans, name)
+
+
+@pytest.mark.parametrize("c2w,rel,rot,trans", REFERENCE_CASES)
+def test_quaternion_pose_model_matches_reference_module(c2w, rel, rot, trans):
+    gold = np.load(GOLDEN)
+    ours = quaternion_pose_run(QuaternionsPoseParameters, c2w, rel, rot, trans)
+    for name in ("rot_embedding", "w2c", "c2w"):
+        ref = torch.from_numpy(gold[pose_golden_key(c2w, rel, rot, trans, name)])
+        assert ours[name].shape == ref.shape and torch.allclose(ours[name], ref, atol=1e-6), name

@@ -1,9 +1,17 @@
-"""RaySamplingStrategy / sample_rays mirrors (sparf_b200/sampling_strategies.py) against the reference's own classes
-(oracle/ref_loader.py): same pools, same torch.randperm draws in the same order => identical rays under one seed."""
+"""RaySamplingStrategy / sample_rays mirrors (sparf_b200/sampling_strategies.py) against the reference's own classes:
+same pools, same torch.randperm draws in the same order => identical rays under one seed.  The rays the reference drew
+on the inputs below are stored in golden/reference_modules.npz (tests/golden/make_module_golden.py regenerates it)."""
+import os
+
+import numpy as np
 import pytest
 import torch
 
 import common
+
+GOLDEN = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "reference_modules.npz")
+CASES = [dict(), dict(sampled_fraction_in_center=0.25), dict(depth_patch=0), dict(depth_patch=0, sampled_fraction_in_center=0.5)]
+SAMPLE_RAYS_KW = [dict(nbr=50), dict(nbr=64, fraction_in_center=0.25), dict()]
 
 
 def _opt(**kw):
@@ -19,31 +27,30 @@ def _opt(**kw):
     return opt
 
 
-@pytest.mark.parametrize("case", [dict(), dict(sampled_fraction_in_center=0.25), dict(depth_patch=0),
-                                  dict(depth_patch=0, sampled_fraction_in_center=0.5)])
+def ray_sampling_run(strategy_cls, sample_rays, case):
+    """Rays drawn by `strategy_cls` (a RaySamplingStrategy) and by `sample_rays` under fixed seeds."""
+    opt = _opt(**case)
+    data = common.make_scene(3, 3, 24, 32)
+    strategy = strategy_cls(opt, data_dict=data, device=torch.device("cpu"))
+    out = {}
+    for center in (False, True):
+        torch.manual_seed(5)
+        out["strategy_center%d" % center] = strategy(96, sample_in_center=center)
+    for i, kw in enumerate(SAMPLE_RAYS_KW):
+        torch.manual_seed(9)
+        out["sample_rays%d_pixels" % i], out["sample_rays%d_rays" % i] = sample_rays(24, 32, **kw)
+    return out
+
+
+def sampling_golden_key(case_index, name):
+    return "sampling_case%d_%s" % (case_index, name)
+
+
+@pytest.mark.parametrize("case", CASES)
 def test_ray_sampling_strategy_matches_reference(case):
-    from oracle import ref_loader
-    if not ref_loader.ref_root():
-        pytest.skip("reference not available")
-    ref = ref_loader.load("trainer")
-    try:
-        from sparf_b200.sampling_strategies import RaySamplingStrategy, sample_rays
-        opt = _opt(**case)
-        data = common.make_scene(3, 3, 24, 32)
-        dev = torch.device("cpu")
-        ours = RaySamplingStrategy(opt, data, dev)
-        theirs = ref.sampling.RaySamplingStrategy(opt, data_dict=data, device=dev)
-        for center in (False, True):
-            torch.manual_seed(5)
-            a = ours(96, sample_in_center=center)
-            torch.manual_seed(5)
-            b = theirs(96, sample_in_center=center)
-            assert a.shape == b.shape and torch.equal(a, b)
-        for kw in (dict(nbr=50), dict(nbr=64, fraction_in_center=0.25), dict()):
-            torch.manual_seed(9)
-            pa, ra = sample_rays(24, 32, **kw)
-            torch.manual_seed(9)
-            pb, rb = ref.sampling.sample_rays(24, 32, **kw)
-            assert torch.equal(pa, pb) and torch.equal(ra, rb)
-    finally:
-        ref_loader._purge()
+    from sparf_b200.sampling_strategies import RaySamplingStrategy, sample_rays
+    gold = np.load(GOLDEN)
+    ours = ray_sampling_run(RaySamplingStrategy, sample_rays, case)
+    for name, a in ours.items():
+        b = torch.from_numpy(gold[sampling_golden_key(CASES.index(case), name)])
+        assert a.shape == b.shape and torch.equal(a, b), name

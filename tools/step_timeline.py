@@ -21,7 +21,7 @@ def main():
     sparf_b200.set_engine(sys.argv[2] if len(sys.argv) > 2 else "auto")
     dev = torch.device("cuda")
     cfg = bench.CONFIGS[cfg_name]
-    pr = bench.build_problem(cfg_name, "ours", dev, seed=0)
+    pr = bench.build_problem(cfg_name, dev, seed=0)
     pr.net.device_side_rng = True
     pr.loss_module.check_finite = False
     fg = FlatGradients(pr.modules)
