@@ -23,13 +23,6 @@
  * sparf_mlp_backward* runs its small CUDA-core reductions beside the weight-gradient kernel (fork after the dgrad
  * chain, join before the call returns control of `stream`: callers see ordinary stream order, and the pattern is
  * capturable into a CUDA graph).  A workspace must not be shared by calls running concurrently on different streams.
- * Environment knobs, read once, for A/B timing only (defaults are the measured-fastest settings):
- *   SPARF_TC_OVERLAP=0   no side stream (everything on `stream`)
- *   SPARF_TC_OVERLAP_BWD=0   only the backward's leftovers back on `stream` (the forward's packing stays on the side stream)
- *   SPARF_TC_TMEMA=0     chain kernels with shared-memory A operands (round-1 generation; also serves the single-pass
- *                        engine and the recompute backward)
- *   SPARF_TC_BWD_SPLIT=n, SPARF_TC_BWD_ND=k   backward pipelined in n sub-chunks, dgrad on k SMs beside wgrad (off)
- *   SPARF_TC_WCOPIES=n   replicas of the packed forward weight stream (L2 hot-spot experiment)
  */
 #ifndef SPARF_B200_H_
 #define SPARF_B200_H_

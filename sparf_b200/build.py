@@ -65,13 +65,13 @@ def _stale() -> bool:
 TRACE_LIB_PATH = os.path.join(LIB_DIR, "libsparf_b200_trace.so")   # debug build (tools/trace_chain.py), never loaded by default
 
 
-def build(force: bool = False, verbose: bool = False, trace: bool = False, variant: str = "", defines_extra=()) -> str:
+def build(force: bool = False, verbose: bool = False, trace: bool = False) -> str:
     """Compile every .cu under csrc/ into one shared library.  Returns its path.  trace=True builds the wait-time
-    tracing variant (-DSPARF_TC_TRACE) next to it; `SPARF_B200_LIB=<path>` makes sparf_b200._lib load that instead."""
+    tracing variant (-DSPARF_TC_TRACE, plus any extra -D flags in SPARF_NVCC_DEFINES) next to it;
+    `SPARF_B200_LIB=<path>` makes sparf_b200._lib load that instead.  The main library takes no defines from the
+    environment: it is built from exactly what _source_hash() covers."""
     out_path = TRACE_LIB_PATH if trace else LIB_PATH
-    if variant:     # experiment builds: lib/libsparf_b200_<variant>.so with extra -D flags (tools only, via SPARF_B200_LIB)
-        out_path = os.path.join(LIB_DIR, "libsparf_b200_%s.so" % variant)
-    if not trace and not variant and not force and not _stale():
+    if not trace and not force and not _stale():
         return LIB_PATH
     os.makedirs(LIB_DIR, exist_ok=True)
     # one builder at a time (several ranks of one job may get here together); whoever waited re-checks first
@@ -79,21 +79,19 @@ def build(force: bool = False, verbose: bool = False, trace: bool = False, varia
     lock = open(os.path.join(LIB_DIR, ".build.lock"), "w")
     fcntl.flock(lock, fcntl.LOCK_EX)
     try:
-        if not trace and not variant and not force and not _stale():
+        if not trace and not force and not _stale():
             return LIB_PATH
-        return _build_locked(out_path, verbose, trace, defines_extra, main_lib=not trace and not variant)
+        return _build_locked(out_path, verbose, trace)
     finally:
         fcntl.flock(lock, fcntl.LOCK_UN)
         lock.close()
 
 
-def _build_locked(out_path, verbose, trace, defines_extra, main_lib):
+def _build_locked(out_path, verbose, trace):
     srcs = sources()
     defines = ["-DSPARF_WITH_TC"] if os.path.exists(os.path.join(CSRC, "mlp_tc.cu")) else []
-    defines += os.environ.get("SPARF_NVCC_DEFINES", "").split()   # extra debug defines
-    if trace:
-        defines.append("-DSPARF_TC_TRACE")
-    defines += list(defines_extra)
+    if trace:   # debug build: extra defines (e.g. -DSPARF_TC_TRACE_EVENTS) from the environment
+        defines += ["-DSPARF_TC_TRACE"] + os.environ.get("SPARF_NVCC_DEFINES", "").split()
     tmp = "%s.tmp.%d" % (out_path, os.getpid())
     cmd = [_nvcc()] + NVCC_FLAGS + defines + ["-I", INCLUDE, "-o", tmp] + srcs
     if verbose:
@@ -106,14 +104,11 @@ def _build_locked(out_path, verbose, trace, defines_extra, main_lib):
     if verbose:
         print(res.stdout + res.stderr)
     os.replace(tmp, out_path)
-    if main_lib:
+    if not trace:
         with open(HASH_PATH, "w") as f:
             f.write(_source_hash())
     return out_path
 
 
 if __name__ == "__main__":
-    _variant = sys.argv[sys.argv.index("--variant") + 1] if "--variant" in sys.argv else ""
-    _defs = sys.argv[sys.argv.index("--defines") + 1].split() if "--defines" in sys.argv else []
-    print(build(force="--force" in sys.argv, verbose="-v" in sys.argv, trace="--trace" in sys.argv, variant=_variant,
-                defines_extra=_defs))
+    print(build(force="--force" in sys.argv, verbose="-v" in sys.argv, trace="--trace" in sys.argv))

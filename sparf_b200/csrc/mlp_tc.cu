@@ -13,8 +13,8 @@
 //                                 -> tcgen05.st -> the MMA warp starts the next layer on that K block; density row,
 //                                 colour head (128 -> 3) and activations in fp32 on CUDA cores
 //   warp 19     image store     : bulk-copies the staged bf16 tape / gradient images from shared memory to HBM
-// Older variants stay for the shapes the TMEM kernels do not cover and for comparison: operands in shared memory with
-// two N128 issuer warps (warps 1 and 18).
+// The forward keeps the older generation for the calls the TMEM kernel does not serve (single-pass engine, bf16
+// recompute forward of the backward): operands in shared memory with two N128 issuer warps (warps 1 and 18).
 //
 // BACKWARD (tc_mlp_backward_tape; tc_mlp_backward re-runs the forward in bf16 "save" mode first):
 //   1. the taped forward dumped every layer's A-operand image (bf16 hi | lo) and 64-bit ReLU masks,
@@ -54,8 +54,6 @@ constexpr int kNumLayers = 9;    // forward tensor-core layers: trunk 0..7 + hea
 constexpr int kNumBwdLayers = 8; // backward tensor-core layers
 constexpr int kTileM = 128;
 constexpr int kStages = 3;         // weight-ring stages of the shared-memory-operand forward kernel
-constexpr int kBwdStages = 6;      // ... of the shared-memory-operand dgrad kernel (its ring takes the encoder blocks, the
-                                   // forward ring and the bias / small-weight tables it does not use)
 constexpr int kMaxStages = 10;
 constexpr int kChunkBytes = 16384;  // one [128 x 64] 16-bit operand block
 constexpr int kEpiWarps = 16;       // 4 TMEM lane quadrants x 4 column quarters of every 64-column block
@@ -90,8 +88,6 @@ constexpr int kOffBar = kOffPart + 3 * 128 * 4 * 4;      // mbarriers
 constexpr int kMaxSlots = 8;                              // image staging slots (g_ready / s_free barrier pairs)
 constexpr int kNumBars = 2 * kMaxStages + 5 + 4 + 2 * kMaxSlots;
 constexpr int kSmemBytes = kOffBar + kNumBars * 8 + 16;
-constexpr int kOffBarBwd = kOffEnc + kBwdStages * kChunkBytes;   // dgrad: barriers right after its ring
-static_assert(kOffBarBwd + kNumBars * 8 + 16 <= kSmemBytes, "dgrad shared-memory map exceeds the launch size");
 static_assert(kSmemBytes + 1024 <= 232448, "shared memory budget exceeded");
 
 // ---- saved operand images (HBM): tensor t, tile, 64-column block, part (hi | lo): 16 KB each
@@ -131,7 +127,6 @@ struct FwdParams {
   int S;
   int num_tiles;
   int passes;              // 3 (compensated) or 1
-  int ncopies;             // replicas of the packed weight stream
   int save;                // dump A-operand images: 0 no, 1 (hi, lo) halves, 2 hi halves only (SPARF_ENGINE_TC_3X_W1)
   Images img;
 };
@@ -175,7 +170,6 @@ struct PackParams {
 template <bool kF16>
 __global__ void pack_weights_kernel(PackParams pp) {
   int chunk = blockIdx.x;
-  pp.packed += (size_t)blockIdx.y * kChunksPerTile * kChunkBytes;   // replica index (spreads the L2 hot spot)
   int l = 0, base = 0;
   for (;; ++l) {
     int n = layer_nkb(l) * layer_nh(l) * 2;
@@ -436,7 +430,9 @@ __device__ __forceinline__ void chain_producer(const ChainSmem& s, const uint8_t
   if ((threadIdx.x & 31) == 0) trace_end(tr, 0);
 }
 
-// Same stream in 32 KB copies over stage pairs (s, s + 1): barriers of the EVEN stage only (kRingPairs).
+// Same stream in 32 KB copies over stage pairs (s, s + 1): barriers of the EVEN stage only.  The TMEM-operand kernels
+// use it: half the copy issues, expect_tx arms, barrier polls and commits per unit of tensor work (inference forward
+// 335 -> 324 us, dgrad 307 -> 302 us against 16 KB copies, profiles/r02_notes.md).
 __device__ __forceinline__ void chain_producer_pairs(const ChainSmem& s, const uint8_t* packed, int my_tiles, int nchunks) {
   Trace tr; trace_begin(tr);
   const int npairs = nchunks / 2, nring = s.nstages / 2;
@@ -506,18 +502,16 @@ __device__ __forceinline__ void chain_issue_block(const ChainSmem& s, uint32_t& 
   }
 }
 
-// N = 256 variant for rings whose chunk order is (K block, part, N half) and whose stage count is even: the two N
+// N = 256 variant for rings whose chunk order is (K block, part, N half), filled by chain_producer_pairs: the two N
 // halves of a part sit in adjacent stages, i.e. form one [256 x 64] K-major operand, and ONE M128 x N256 MMA covers
 // them.  Half the instructions and barrier round trips per unit of tensor work (one issuer warp suffices) and
 // 96 instead of 128 B/clk of shared-memory operand fetch.
-template <bool kBig = false>
 __device__ __forceinline__ void chain_issue_pair256(const ChainSmem& s, uint32_t& stage, uint32_t& phase, uint32_t a_hi,
                                                     uint32_t a_lo, uint32_t d_addr, uint32_t idesc, bool first_kb, Trace& tr) {
   const uint32_t ring_addr = smem_u32(s.ring);
   for (int part = 0; part < 2; ++part) {
     long long t0 = trace_tic();
-    if (kBig) mbar_wait(&s.w_full[stage], phase);
-    else mbar_wait_two(&s.w_full[stage], phase, &s.w_full[stage + 1], phase);
+    mbar_wait(&s.w_full[stage], phase);
     trace_toc(tr, 2, t0);
     tc_fence_after();
     const uint64_t db0 = make_smem_desc(ring_addr) + (uint64_t)(stage * (kChunkBytes >> 4));
@@ -531,7 +525,6 @@ __device__ __forceinline__ void chain_issue_pair256(const ChainSmem& s, uint32_t
         if (part == 0) umma_ss(d_addr, dal0 + (uint64_t)(2 * ks), db, idesc, 1u);
       }
       umma_commit(&s.w_empty[stage]);
-      if (!kBig) umma_commit(&s.w_empty[stage + 1]);
     }
     __syncwarp();
     stage += 2;
@@ -542,14 +535,12 @@ __device__ __forceinline__ void chain_issue_pair256(const ChainSmem& s, uint32_t
 // Same with the A operand in tensor memory (columns a_hi_t / a_lo_t of this K block, +8 columns per K16 step): the MMA
 // fetches only B from shared memory and the epilogue hands activations over with tcgen05.st instead of swizzled
 // st.shared + fence.proxy.async.
-template <bool kBig = false>
 __device__ __forceinline__ void chain_issue_pair256_ts(const ChainSmem& s, uint32_t& stage, uint32_t& phase, uint32_t a_hi_t,
                                                        uint32_t a_lo_t, uint32_t d_addr, uint32_t idesc, bool first_kb, Trace& tr) {
   const uint32_t ring_addr = smem_u32(s.ring);
   for (int part = 0; part < 2; ++part) {
     long long t0 = trace_tic();
-    if (kBig) mbar_wait(&s.w_full[stage], phase);
-    else mbar_wait_two(&s.w_full[stage], phase, &s.w_full[stage + 1], phase);
+    mbar_wait(&s.w_full[stage], phase);
     trace_toc(tr, 2, t0);
     tc_fence_after();
     // descriptor of K step ks = descriptor of the stage + 2 ks in its 16-byte start-address field (no carry: the ring
@@ -564,7 +555,6 @@ __device__ __forceinline__ void chain_issue_pair256_ts(const ChainSmem& s, uint3
         if (part == 0) umma_ts(d_addr, a_lo_t + ks * 8, db, idesc, 1u);
       }
       umma_commit(&s.w_empty[stage]);
-      if (!kBig) umma_commit(&s.w_empty[stage + 1]);
     }
     __syncwarp();
     stage += 2;
@@ -572,50 +562,30 @@ __device__ __forceinline__ void chain_issue_pair256_ts(const ChainSmem& s, uint3
   }
 }
 
-// one [128 x 64] weight chunk per part against an A operand in tensor memory (the N = 128 colour-head layer)
-template <bool kBig = false>
+// one [128 x 64] weight chunk against an A operand in tensor memory (the N = 128 colour-head layer): its (hi, lo) parts
+// arrive together in the stage pair (stage, stage + 1)
 __device__ __forceinline__ void chain_issue_single_ts(const ChainSmem& s, uint32_t& stage, uint32_t& phase, uint32_t a_hi_t,
                                                       uint32_t a_lo_t, uint32_t d_addr, uint32_t idesc, bool first_kb, Trace& tr) {
   const uint32_t ring_addr = smem_u32(s.ring);
-  if (kBig) {     // (hi, lo) parts of the chunk arrived together in the stage pair (stage, stage + 1)
-    twait(tr, 2, &s.w_full[stage], phase);
-    tc_fence_after();
-    const uint64_t db0 = make_smem_desc(ring_addr) + (uint64_t)(stage * (kChunkBytes >> 4));
-    if (elect_one()) {
+  twait(tr, 2, &s.w_full[stage], phase);
+  tc_fence_after();
+  const uint64_t db0 = make_smem_desc(ring_addr) + (uint64_t)(stage * (kChunkBytes >> 4));
+  if (elect_one()) {
 #pragma unroll
-      for (int part = 0; part < 2; ++part) {
-#pragma unroll
-        for (int ks = 0; ks < 4; ++ks) {
-          const uint64_t db = db0 + (uint64_t)(part * (kChunkBytes >> 4) + 2 * ks);
-          const uint32_t acc = (first_kb && part == 0 && ks == 0) ? 0u : 1u;
-          umma_ts(d_addr, a_hi_t + ks * 8, db, idesc, acc);
-          if (part == 0) umma_ts(d_addr, a_lo_t + ks * 8, db, idesc, 1u);
-        }
-      }
-      umma_commit(&s.w_empty[stage]);
-    }
-    __syncwarp();
-    stage += 2;
-    if (stage == (uint32_t)s.nstages) { stage = 0; phase ^= 1; }
-    return;
-  }
-  for (int part = 0; part < 2; ++part) {
-    twait(tr, 2, &s.w_full[stage], phase);
-    tc_fence_after();
-    const uint64_t db0 = make_smem_desc(ring_addr) + (uint64_t)(stage * (kChunkBytes >> 4));
-    if (elect_one()) {
+    for (int part = 0; part < 2; ++part) {
 #pragma unroll
       for (int ks = 0; ks < 4; ++ks) {
-        const uint64_t db = db0 + (uint64_t)(2 * ks);
+        const uint64_t db = db0 + (uint64_t)(part * (kChunkBytes >> 4) + 2 * ks);
         const uint32_t acc = (first_kb && part == 0 && ks == 0) ? 0u : 1u;
         umma_ts(d_addr, a_hi_t + ks * 8, db, idesc, acc);
         if (part == 0) umma_ts(d_addr, a_lo_t + ks * 8, db, idesc, 1u);
       }
-      umma_commit(&s.w_empty[stage]);
     }
-    __syncwarp();
-    if (++stage == (uint32_t)s.nstages) { stage = 0; phase ^= 1; }
+    umma_commit(&s.w_empty[stage]);
   }
+  __syncwarp();
+  stage += 2;
+  if (stage == (uint32_t)s.nstages) { stage = 0; phase ^= 1; }
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -628,73 +598,26 @@ __device__ __forceinline__ void chain_issue_single_ts(const ChainSmem& s, uint32
 // One issuer warp (M128 x N256 MMAs over paired ring stages), the epilogue drains its whole share of the accumulator
 // into registers and frees it at once; warp 19 streams the tape images out of the staging slots with bulk copies.
 // Image staging (taped forward: kFwdSlots x 16 KB, one (block, part) each; dgrad: kDgSlots x 32 KB, one block's hi | lo).
-// The store warp keeps up to kStoreInflight bulk stores in flight: a slot is handed back to the epilogue warps when the
-// store issued kStoreInflight - 1 steps later has been committed and `cp.async.bulk.wait_group.read` reports its
-// predecessors' sources read.  Measured (profiles/r02_notes.md): one store at a time costs ~1000 clk per 16 KB copy and
-// the epilogue warps wait 12 % (forward) / 19 % (dgrad) of the kernel for a free slot -- yet trading ring stages for
-// slots (forward 5 slots + 6 stages, dgrad 3 + 8) or keeping 2-3 stores in flight measured SLOWER (taped forward 435 ->
-// 453..461 us, dgrad 291 -> 312..370 us): the weight ring's depth is worth more than the slots.  Defaults = 3 / 8, 2 / 10, 1.
-#ifndef SPARF_FWD_SLOTS
-#define SPARF_FWD_SLOTS 3
-#endif
-#ifndef SPARF_FWD_RING
-#define SPARF_FWD_RING 8
-#endif
-#ifndef SPARF_DG_SLOTS
-#define SPARF_DG_SLOTS 2
-#endif
-#ifndef SPARF_DG_RING
-#define SPARF_DG_RING 10
-#endif
-#ifndef SPARF_STORE_INFLIGHT
-#define SPARF_STORE_INFLIGHT 1
-#endif
-constexpr int kFwdSlots = SPARF_FWD_SLOTS, kDgSlots = SPARF_DG_SLOTS, kStoreInflight = SPARF_STORE_INFLIGHT;
-static_assert(kFwdSlots <= kMaxSlots && kDgSlots <= kMaxSlots && kStoreInflight >= 1 && kStoreInflight < kFwdSlots &&
-              kStoreInflight < kDgSlots, "staging slots / stores in flight");
-template <int N> __device__ __forceinline__ void bulk_wait_read() { asm volatile("cp.async.bulk.wait_group.read %0;" ::"n"(N) : "memory"); }
-// SPARF_STORE_LSU = 1 (experiment, default off): the store warp(s) copy a staged block to HBM with ordinary 16-byte
-// loads / stores (ld.shared -> st.global, 512 contiguous bytes per warp instruction) instead of a bulk copy, and the
-// epilogue warps drop their generic -> async proxy fence.  Measured SLOWER (profiles/r02_notes.md): a warp needs
-// ~1190 clk per 16 KB block this way (the bulk copy: ~1040) because it shares issue slots and the LSU with the epilogue
-// warps; taped forward 427 -> 436 us, dgrad 306 -> 337 us.
-#ifndef SPARF_STORE_LSU
-#define SPARF_STORE_LSU 0
-#endif
-constexpr bool kStoreLsu = SPARF_STORE_LSU != 0;
-// SPARF_RING_PAIRS = 1 (TMEM-operand kernels): the weight producer moves one 32 KB [256 x 64] operand (or the
-// (hi, lo) parts of a [128 x 64] colour-head chunk) per bulk copy and mbarrier instead of two 16 KB chunks: half the
-// copy issues, expect_tx arms, barrier polls and commits per unit of tensor work (inference forward 335 -> 324 us,
-// dgrad 307 -> 302 us, taped forward unchanged).
-#ifndef SPARF_RING_PAIRS
-#define SPARF_RING_PAIRS 1
-#endif
-constexpr bool kRingPairs = SPARF_RING_PAIRS != 0;
-// LSU mode: number of store warps (1: warp 19; 2: + warp 18, the second-issuer warp the TMEM-operand kernels leave idle);
-// store warp i takes the staged blocks with running index % kStoreWarps == i
-#ifndef SPARF_STORE_WARPS
-#define SPARF_STORE_WARPS 2
-#endif
-constexpr int kStoreWarps = kStoreLsu ? SPARF_STORE_WARPS : 1;
-// whole warp: copy `bytes` (multiple of 4096) from shared to global memory, streaming stores
-__device__ __forceinline__ void warp_copy_s2g(uint8_t* gdst, const uint8_t* ssrc, int bytes, int lane) {
-  const uint4* src = reinterpret_cast<const uint4*>(ssrc) + lane;
-  uint4* dst = reinterpret_cast<uint4*>(gdst) + lane;
-  for (int i = 0; i < bytes / 512; i += 8) {
-    uint4 v[8];
-#pragma unroll
-    for (int u = 0; u < 8; ++u) v[u] = src[(i + u) * 32];
-#pragma unroll
-    for (int u = 0; u < 8; ++u) __stcs(dst + (i + u) * 32, v[u]);
-  }
-}
+// The store warp keeps one bulk store in flight: it hands a slot back to the epilogue warps as soon as
+// `cp.async.bulk.wait_group.read 0` reports the slot read.  Measured (profiles/r02_notes.md): one store at a time costs
+// ~1000 clk per 16 KB copy and the epilogue warps wait 12 % (forward) / 19 % (dgrad) of the kernel for a free slot --
+// yet trading ring stages for slots (forward 5 slots + 6 stages, dgrad 3 + 8) or keeping 2-3 stores in flight measured
+// SLOWER (taped forward 435 -> 453..461 us, dgrad 291 -> 312..370 us): the weight ring's depth is worth more than the
+// slots.  So did copying with ld.shared / st.global instead of bulk copies (taped forward 427 -> 436 us, dgrad 306 ->
+// 337 us): the store warp then shares issue slots and the LSU with the epilogue warps.
+constexpr int kFwdSlots = 3, kDgSlots = 2;
+static_assert(kFwdSlots <= kMaxSlots && kDgSlots <= kMaxSlots, "staging slots");
 constexpr int kOffEncT = 0;
 constexpr int kOffStgT = 2 * kChunkBytes;
-constexpr int kOffRingTSave = kOffStgT + kFwdSlots * kChunkBytes, kStagesTSave = SPARF_FWD_RING;
-static_assert(kStagesTSave % 2 == 0 && SPARF_DG_RING % 2 == 0, "N = 256 MMAs pair adjacent ring stages");
+constexpr int kOffRingTSave = kOffStgT + kFwdSlots * kChunkBytes, kStagesTSave = 8;
 constexpr int kOffRingTInf = 2 * kChunkBytes, kStagesTInf = 10;
+// dgrad: the staging slots, a 10-stage ring (5 [256 x 64] operands), the barriers right after it
+constexpr int kOffRingDg = kOffAct + kDgSlots * 2 * kChunkBytes, kStagesDg = 10;
+constexpr int kOffBarBwd = kOffRingDg + kStagesDg * kChunkBytes;
+static_assert(kStagesTSave % 2 == 0 && kStagesTInf % 2 == 0 && kStagesDg % 2 == 0, "N = 256 MMAs pair adjacent ring stages");
 static_assert(kOffRingTSave + kStagesTSave * kChunkBytes <= kOffBias && kOffRingTInf + kStagesTInf * kChunkBytes <= kOffBias,
               "tensor-memory-operand forward: shared-memory map");
+static_assert(kOffBarBwd + kNumBars * 8 + 16 <= kSmemBytes, "dgrad shared-memory map exceeds the launch size");
 
 // kHiTape (with kTmemA, p.save == 2): the tape images get their bf16 hi halves only (SPARF_ENGINE_TC_3X_W1)
 template <bool kF16, bool kTmemA = false, bool kHiTape = false>
@@ -724,7 +647,6 @@ __global__ void __launch_bounds__(kThreads, 1) tc_mlp_fwd_kernel(const FwdParams
     s_misc[1] = p.b9[0]; s_misc[2] = p.b9[1]; s_misc[3] = p.b9[2];
   }
   if (tid < 16) s_misc[8 + tid] = tid < kL ? band_weight(p.c2f, kL, tid) : 0.f;
-  const uint8_t* my_packed = p.packed + (size_t)(blockIdx.x % p.ncopies) * kChunksPerTile * kChunkBytes;
   if (tid == 32) chain_init_barriers(cs, kTmemA ? 1 : kIssuers);
   if (warp == 1) {
     tmem_alloc(cs.tmem_slot, 512);
@@ -738,9 +660,9 @@ __global__ void __launch_bounds__(kThreads, 1) tc_mlp_fwd_kernel(const FwdParams
   const int my_tiles = (p.num_tiles - (int)blockIdx.x + (int)gridDim.x - 1) / (int)gridDim.x;   // tiles b, b + grid, ...
 
   if (warp == 0) {
-    if (kTmemA && kRingPairs) chain_producer_pairs(cs, my_packed, my_tiles, kChunksPerTile);
-    else chain_producer(cs, my_packed, my_tiles, kChunksPerTile, p.passes == 1);
-  } else if (warp == 1 || (warp == 2 + kEpiWarps && !(kTmemA && kStoreWarps == 2))) {
+    if (kTmemA) chain_producer_pairs(cs, p.packed, my_tiles, kChunksPerTile);
+    else chain_producer(cs, p.packed, my_tiles, kChunksPerTile, p.passes == 1);
+  } else if (warp == 1 || warp == 2 + kEpiWarps) {
     const int issuer = warp == 1 ? 0 : 1;
     // ============================== MMA issuer ==============================
     if (kTmemA) {
@@ -761,15 +683,15 @@ __global__ void __launch_bounds__(kThreads, 1) tc_mlp_fwd_kernel(const FwdParams
               if (kb_is_enc(l, kbi)) {                              // encoder block: operand in shared memory
                 if (l == 0) { twait(tr, 1, &cs.a_ready[4], a_cnt[4] & 1); ++a_cnt[4]; }
                 tc_fence_after();
-                chain_issue_pair256<kRingPairs>(cs, stage, phase, enc_addr, enc_addr + kChunkBytes, tmem_base, idesc256, kbi == 0, tr);
+                chain_issue_pair256(cs, stage, phase, enc_addr, enc_addr + kChunkBytes, tmem_base, idesc256, kbi == 0, tr);
               } else {
                 const int a = kb_act_index(l, kbi);
                 twait(tr, 1, &cs.a_ready[a], a_cnt[a] & 1);
                 ++a_cnt[a];
                 tc_fence_after();
                 const uint32_t a_hi_t = tmem_base + 256u + (uint32_t)(a * 32), a_lo_t = tmem_base + 384u + (uint32_t)(a * 32);
-                if (l == 8) chain_issue_single_ts<kRingPairs>(cs, stage, phase, a_hi_t, a_lo_t, tmem_base, idesc128, kbi == 0, tr);
-                else chain_issue_pair256_ts<kRingPairs>(cs, stage, phase, a_hi_t, a_lo_t, tmem_base, idesc256, kbi == 0, tr);
+                if (l == 8) chain_issue_single_ts(cs, stage, phase, a_hi_t, a_lo_t, tmem_base, idesc128, kbi == 0, tr);
+                else chain_issue_pair256_ts(cs, stage, phase, a_hi_t, a_lo_t, tmem_base, idesc256, kbi == 0, tr);
               }
             }
             if (elect_one()) umma_commit(&cs.d_full[0]);
@@ -815,9 +737,8 @@ __global__ void __launch_bounds__(kThreads, 1) tc_mlp_fwd_kernel(const FwdParams
       if (lane == 0 && issuer == 0) trace_end(tr, 1);
     }
   } else if (kTmemA && warp >= 2 + kEpiWarps) {
-    // ============================== tape store warp(s) ==============================
+    // ============================== tape store warp (warp 19) ==============================
     // stream the bf16 tape images of layers 0..7 out of the rotating staging slots (one 16 KB block each)
-    const uint32_t store_id = (uint32_t)(2 + kEpiWarps + kIssuers - 1 - warp);   // warp 19 -> 0, warp 18 -> 1
     if (p.save) {
       uint8_t* stg = smem + kOffStgT;
       constexpr int nparts = kHiTape ? 1 : 2;
@@ -829,29 +750,23 @@ __global__ void __launch_bounds__(kThreads, 1) tc_mlp_fwd_kernel(const FwdParams
           for (int jq = 0; jq < 4 * nparts; ++jq) {                // (block j, part)
             const int jp = nparts == 2 ? jq : 2 * jq;
             const uint32_t qs = (uint32_t)nparts * (32u * (uint32_t)it + 4u * (uint32_t)l) + (uint32_t)jq;
-            if (qs % (uint32_t)kStoreWarps != store_id) continue;
             const uint32_t slot = qs % (uint32_t)kFwdSlots, k = qs / (uint32_t)kFwdSlots;
             twait(tr, 0, &cs.g_ready[slot], k & 1);
             long long t0 = trace_tic();
-            if (kStoreLsu) {
-              warp_copy_s2g(p.img.at(t_img, tile, jp >> 1, jp & 1), stg + (size_t)slot * kChunkBytes, kChunkBytes, lane);
-              __syncwarp();
-              if (lane == 0) mbar_arrive(&cs.s_free[slot]);
-            } else if (elect_one()) {
+            if (elect_one()) {
               bulk_s2g(p.img.at(t_img, tile, jp >> 1, jp & 1), stg + (size_t)slot * kChunkBytes, kChunkBytes);
               bulk_commit_group();
-              bulk_wait_read<kStoreInflight - 1>();      // every store but the newest kStoreInflight - 1 has read its slot
-              if (qs + 1u >= (uint32_t)kStoreInflight)
-                mbar_arrive(&cs.s_free[(qs + 1u - (uint32_t)kStoreInflight) % (uint32_t)kFwdSlots]);
+              bulk_wait_read_all();
+              mbar_arrive(&cs.s_free[slot]);
             }
             __syncwarp();
             trace_toc(tr, 1, t0);
           }
         }
       }
-      if (!kStoreLsu && elect_one()) bulk_wait_all();
+      if (elect_one()) bulk_wait_all();
       __syncwarp();
-      if (lane == 0 && store_id == 0) trace_end(tr, 4);
+      if (lane == 0) trace_end(tr, 4);
     }
   } else if (warp < 2 + kEpiWarps) {
     // ============================== epilogue warps ==============================
@@ -985,7 +900,7 @@ __global__ void __launch_bounds__(kThreads, 1) tc_mlp_fwd_kernel(const FwdParams
                   const uint32_t slot = qs % (uint32_t)kFwdSlots, k = qs / (uint32_t)kFwdSlots;
                   if (k > 0) twait(tr, 1, &cs.s_free[slot], (k - 1) & 1);
                   store16_part(part == 0 ? sp.hi : sp.lo, row, cq * kEpiCols, stg + (size_t)slot * kChunkBytes);
-                  if (!kStoreLsu) fence_proxy_async_smem();   // (LSU store warp: generic proxy on both sides)
+                  fence_proxy_async_smem();
                   __syncwarp();
                   if (lane == 0) mbar_arrive(&cs.g_ready[slot]);
                 }
@@ -1044,29 +959,6 @@ __global__ void __launch_bounds__(kThreads, 1) tc_mlp_fwd_kernel(const FwdParams
             if (save) {   // hid image for the 128->3 head's weight gradient and its ReLU mask
               split16<false>(f, sp);
               store16_image(sp, row, cq * kEpiCols, p.img.at(T_HID, tile, j, 0), p.img.at(T_HID, tile, j, 1), nparts == 2);
-            }
-          } else if (kTmemA) {
-            split16<kF16>(f, sp);
-            tmem_st8(tmem_base + t_lane + 256u + (uint32_t)(j * 32 + cq * 8), sp.hi);
-            tmem_st8(tmem_base + t_lane + 384u + (uint32_t)(j * 32 + cq * 8), sp.lo);
-            tmem_st_wait();
-            tc_fence_before();
-            __syncwarp();
-            if (lane == 0) mbar_arrive(&cs.a_ready[j]);
-            if (save) {          // bf16 tape image through the staging slots (the store warp bulk-copies them out)
-              if (kF16) split16<false>(f, sp);
-              uint8_t* stg = smem + kOffStgT;
-#pragma unroll
-              for (int part = 0; part < 2; ++part) {
-                if (part >= nparts) break;
-                const uint32_t qs = (uint32_t)nparts * (32u * (uint32_t)it + 4u * (uint32_t)l + (uint32_t)j) + (uint32_t)part;
-                const uint32_t slot = qs % (uint32_t)kFwdSlots, k = qs / (uint32_t)kFwdSlots;
-                if (k > 0) twait(tr, 1, &cs.s_free[slot], (k - 1) & 1);
-                store16_part(part == 0 ? sp.hi : sp.lo, row, cq * kEpiCols, stg + (size_t)slot * kChunkBytes);
-                fence_proxy_async_smem();
-                __syncwarp();
-                if (lane == 0) mbar_arrive(&cs.g_ready[slot]);
-              }
             }
           } else {
             split16<kF16>(f, sp);
@@ -1129,22 +1021,17 @@ __global__ void __launch_bounds__(kThreads, 1) tc_mlp_fwd_kernel(const FwdParams
 // ------------------------------------------------------------------------------------------------
 // the fused input-gradient (dgrad) kernel: dL/dz chain from the colour head to layer 0
 // ------------------------------------------------------------------------------------------------
-// kTmemA: TMEM = [0,256) ONE accumulator | [256,384) A hi | [384,512) A lo (32 columns per K block).
+// TMEM = [0,256) ONE accumulator | [256,384) A hi | [384,512) A lo (32 columns per K block).
 // The epilogue loads its whole share of the accumulator into registers first and hands the accumulator back at once,
-// so a single accumulator still lets layer l+1's MMAs overlap layer l's epilogue.
-template <bool kTmemA>
+// so a single accumulator still lets layer l+1's MMAs overlap layer l's epilogue.  Shared memory holds no A operand:
+// kDgSlots rotating (hi, lo) staging slots for the gradient images' bulk stores, then the weight ring.
 __global__ void __launch_bounds__(kThreads, 1) tc_mlp_dgrad_kernel(const BwdParams p) {
   extern __shared__ uint8_t smem_raw[];
   uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~(uintptr_t)1023);
-  // shared-memory map of this kernel: activations (8 blocks) | 6-stage weight ring | barriers.  The density row and the
-  // 128 -> 3 colour weights (2.5 KB, read by every thread) come from global memory through L1.
+  // The density row and the 128 -> 3 colour weights (2.5 KB, read by every thread) come from global memory through L1.
   const float* __restrict__ s_w7r0 = p.w7;
   const float* __restrict__ s_w9 = p.w9;
-  // kTmemA: the activation blocks are no MMA operands any more, only a staging area for the image stores: two rotating
-  // (hi, lo) block pairs (64 KB) are enough and the weight ring takes the rest: 10 stages = 5 [256 x 64] operands
-  static_assert(kOffAct + kDgSlots * 2 * kChunkBytes + SPARF_DG_RING * kChunkBytes <= kOffBarBwd, "dgrad (TMEM operand) shared-memory map");
-  const ChainSmem cs = kTmemA ? chain_carve(smem, kOffAct + kDgSlots * 2 * kChunkBytes, SPARF_DG_RING, kOffBarBwd)
-                              : chain_carve(smem, kOffEnc, kBwdStages, kOffBarBwd);
+  const ChainSmem cs = chain_carve(smem, kOffRingDg, kStagesDg, kOffBarBwd);
   const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
 
   if (tid == 32) chain_init_barriers(cs, 1);   // ONE issuer warp (N = 256 MMAs)
@@ -1159,94 +1046,61 @@ __global__ void __launch_bounds__(kThreads, 1) tc_mlp_dgrad_kernel(const BwdPara
   const int my_tiles = (p.num_tiles - (int)blockIdx.x + (int)gridDim.x - 1) / (int)gridDim.x;
 
   if (warp == 0) {
-    if (kTmemA && kRingPairs) chain_producer_pairs(cs, p.packed, my_tiles, kBwdChunksPerTile);
-    else chain_producer(cs, p.packed, my_tiles, kBwdChunksPerTile, false);
-  } else if (warp == 1 || (warp == 2 + kEpiWarps && !(kTmemA && kStoreWarps == 2))) {
-    const int issuer = warp == 1 ? 0 : 1;
-    if (issuer == 0) {
+    chain_producer_pairs(cs, p.packed, my_tiles, kBwdChunksPerTile);
+  } else if (warp == 1 || warp == 2 + kEpiWarps) {
+    if (warp == 1) {   // (warp 18 idles)
       const uint32_t idesc = make_idesc(128, 256, 1);
-      const uint32_t act_addr = smem_u32(smem + kOffAct);
       uint32_t stage = 0, phase = 0;
       uint32_t a_cnt[4] = {0, 0, 0, 0};
-      uint32_t d_cnt[2] = {0, 0};
+      uint32_t d_cnt = 0;
       Trace tr; trace_begin(tr);
       for (int it = 0; it < my_tiles; ++it) {
         for (int bl = 0; bl < kNumBwdLayers; ++bl) {
-          const int buf = kTmemA ? 0 : (bl & 1);
-          twait(tr, 0, &cs.d_empty[buf], (d_cnt[buf] & 1) ^ 1);
-          ++d_cnt[buf];
+          twait(tr, 0, &cs.d_empty[0], (d_cnt & 1) ^ 1);
+          ++d_cnt;
           tc_fence_after();
           const int nkb = bwd_nkb(bl);
           for (int kbi = 0; kbi < nkb; ++kbi) {
             twait(tr, 1, &cs.a_ready[kbi], a_cnt[kbi] & 1);
             ++a_cnt[kbi];
             tc_fence_after();
-            if (kTmemA) {
-              chain_issue_pair256_ts<kRingPairs>(cs, stage, phase, tmem_base + 256u + (uint32_t)(kbi * 32),
-                                     tmem_base + 384u + (uint32_t)(kbi * 32), tmem_base, idesc, kbi == 0, tr);
-            } else {
-              const uint32_t a_hi = act_addr + kbi * kChunkBytes, a_lo = act_addr + (4 + kbi) * kChunkBytes;
-              chain_issue_pair256(cs, stage, phase, a_hi, a_lo, tmem_base + (uint32_t)(buf * 256), idesc, kbi == 0, tr);
-            }
+            chain_issue_pair256_ts(cs, stage, phase, tmem_base + 256u + (uint32_t)(kbi * 32),
+                                   tmem_base + 384u + (uint32_t)(kbi * 32), tmem_base, idesc, kbi == 0, tr);
           }
-          if (elect_one()) umma_commit(&cs.d_full[buf]);
+          if (elect_one()) umma_commit(&cs.d_full[0]);
           __syncwarp();
         }
       }
       if (lane == 0) trace_end(tr, 1);
     }
   } else if (warp >= 2 + kEpiWarps) {
-    // ============================== gradient-image store warp(s) ==============================
-    // stream every finished [128 x 64] hi / lo block pair (already in the HBM image layout) out
-    const uint32_t store_id = (uint32_t)(2 + kEpiWarps + kIssuers - 1 - warp);   // warp 19 -> 0, warp 18 (TMEM kernel) -> 1
-    uint8_t* act_hi = smem + kOffAct;
-    uint8_t* act_lo = smem + kOffAct + 4 * kChunkBytes;
+    // ============================== gradient-image store warp (warp 19) ==============================
+    // stream every finished [128 x 64] hi / lo block pair (already in the HBM image layout) out of the staging slots
     for (int it = 0; it < my_tiles; ++it) {
       const int tile = (int)blockIdx.x + it * (int)gridDim.x;
-      const bool tile_ok = tile < p.num_tiles;
       for (int step = 0; step <= kNumBwdLayers; ++step) {          // step 0 = head (blocks 0, 1), step bl + 1 = layer bl
         const int nblk = step == 0 ? 2 : 4;
         const int t_out = step == 0 ? T_GHID : (step == 1 ? T_G7F : t_g(8 - step));
         for (int j = 0; j < nblk; ++j) {
-          // stand-alone blocks: barrier j, write number n of block j.  kTmemA: two rotating staging slots, q = running
-          // index of the (tile, step, block) writes, slot = q & 1, k = q >> 1 its per-slot sequence number
+          // q = running index of the (tile, step, block) writes: slot q % kDgSlots, q / kDgSlots its per-slot number
           const uint32_t q = 34u * (uint32_t)it + (step == 0 ? (uint32_t)j : 2u + 4u * (uint32_t)(step - 1) + (uint32_t)j);
-          const uint32_t n = j < 2 ? 9u * (uint32_t)it + (uint32_t)step : 8u * (uint32_t)it + (uint32_t)step - 1u;
-          if (kTmemA && q % (uint32_t)kStoreWarps != store_id) continue;
-          const int bi = kTmemA ? (int)(q % (uint32_t)kDgSlots) : j;
-          const uint8_t* src_hi = kTmemA ? smem + kOffAct + (size_t)bi * 2 * kChunkBytes : act_hi + (size_t)j * kChunkBytes;
-          const uint8_t* src_lo = kTmemA ? src_hi + kChunkBytes : act_lo + (size_t)j * kChunkBytes;
-          mbar_wait(&cs.g_ready[bi], (kTmemA ? (q / (uint32_t)kDgSlots) : n) & 1);
-          if (kTmemA && kStoreLsu) {
-            if (tile_ok) warp_copy_s2g(p.img.at(t_out, tile, j, 0), src_hi, 2 * kChunkBytes, lane);
-            __syncwarp();
-            if (lane == 0) mbar_arrive(&cs.s_free[bi]);
-          } else if (elect_one()) {
-            if (kTmemA) {
-              // (hi | lo) of a block are adjacent in the slot AND in the HBM image: one 32 KB bulk store.  A dummy tile
-              // (never with stand-alone CTAs) would still need its (empty) group for the in-flight accounting.
-              // hi_only (SPARF_ENGINE_TC_3X_W1): images only the single-pass weight-gradient kernel reads keep their hi half
-              const bool both = !p.hi_only || t_out == T_GHID || step == kNumBwdLayers || t_out == t_g(4);
-              if (tile_ok) bulk_s2g(p.img.at(t_out, tile, j, 0), src_hi, (both ? 2 : 1) * kChunkBytes);
-              bulk_commit_group();
-              bulk_wait_read<kStoreInflight - 1>();
-              if (q + 1u >= (uint32_t)kStoreInflight)
-                mbar_arrive(&cs.s_free[(q + 1u - (uint32_t)kStoreInflight) % (uint32_t)kDgSlots]);
-            } else {
-              if (tile_ok) {
-                bulk_s2g(p.img.at(t_out, tile, j, 0), src_hi, kChunkBytes);
-                bulk_s2g(p.img.at(t_out, tile, j, 1), src_lo, kChunkBytes);
-                bulk_commit_group();
-                bulk_wait_read_all();
-              }
-              mbar_arrive(&cs.s_free[bi]);
-            }
+          const int slot = (int)(q % (uint32_t)kDgSlots);
+          const uint8_t* src = smem + kOffAct + (size_t)slot * 2 * kChunkBytes;
+          mbar_wait(&cs.g_ready[slot], (q / (uint32_t)kDgSlots) & 1);
+          if (elect_one()) {
+            // (hi | lo) of a block are adjacent in the slot AND in the HBM image: one 32 KB bulk store.
+            // hi_only (SPARF_ENGINE_TC_3X_W1): images only the single-pass weight-gradient kernel reads keep their hi half
+            const bool both = !p.hi_only || t_out == T_GHID || step == kNumBwdLayers || t_out == t_g(4);
+            bulk_s2g(p.img.at(t_out, tile, j, 0), src, (both ? 2 : 1) * kChunkBytes);
+            bulk_commit_group();
+            bulk_wait_read_all();
+            mbar_arrive(&cs.s_free[slot]);
           }
           __syncwarp();
         }
       }
     }
-    if (!(kTmemA && kStoreLsu) && elect_one()) bulk_wait_all();
+    if (elect_one()) bulk_wait_all();
     __syncwarp();
   } else {
     const int e = warp - 2;
@@ -1254,17 +1108,13 @@ __global__ void __launch_bounds__(kThreads, 1) tc_mlp_dgrad_kernel(const BwdPara
     const int cq = e >> 2;
     const int row = q * 32 + lane;
     const uint32_t t_lane = (uint32_t)(q * 32) << 16;
-    uint32_t d_cnt[2] = {0, 0};
-    uint8_t* act_hi = smem + kOffAct;
-    uint8_t* act_lo = smem + kOffAct + 4 * kChunkBytes;
+    uint32_t d_cnt = 0;
     Trace tr; trace_begin(tr);
 
     for (int it = 0; it < my_tiles; ++it) {
-      const int tile_raw = (int)blockIdx.x + it * (int)gridDim.x;
-      const bool tile_ok = true;
-      const int tile = tile_raw;
-      const long long m = (long long)tile_raw * kTileM + row;
-      const bool valid = tile_ok && m < p.M;
+      const int tile = (int)blockIdx.x + it * (int)gridDim.x;
+      const long long m = (long long)tile * kTileM + row;
+      const bool valid = m < p.M;
 
       // ---------------- head: g_pre = d_rgb * c (1 - c); g_raw = d_sigma * (1 - e^-sigma) [= sigmoid(z)];
       //                  g_hid = (hid > 0) * (g_pre . W9)  -> A blocks 0, 1
@@ -1280,9 +1130,8 @@ __global__ void __launch_bounds__(kThreads, 1) tc_mlp_dgrad_kernel(const BwdPara
           *reinterpret_cast<float4*>(p.g_pre + m * 4) = make_float4(gp0, gp1, gp2, 0.f);
         }
       }
-      // Shared-memory block j is both the next layer's A operand and the source of the gradient image's bulk store
-      // (store warp below); write number n of a block must wait for the store of write n - 1 to have read it.
-      //   blocks 0, 1: n = 9 * it + (head: 0 | layer bl: bl + 1);   blocks 2, 3: n = 8 * it + bl
+      // Every gradient block goes to tensor memory (the next layer's A operand) and through a staging slot to the store
+      // warp; write number k of a slot waits for the store of write k - 1 to have read it (qs numbered as in the store warp)
       const uint2 hid_mask = *p.img.mask_at(tile, 8, row, cq);
 #pragma unroll 1
       for (int j = 0; j < 2; ++j) {
@@ -1296,83 +1145,55 @@ __global__ void __launch_bounds__(kThreads, 1) tc_mlp_dgrad_kernel(const BwdPara
         }
         Split16 sp;
         split16<false>(f, sp);
-        if (kTmemA) {   // operand for the MMA: tensor memory; the shared-memory copy below only feeds the image store
-          tmem_st8(tmem_base + t_lane + 256u + (uint32_t)(j * 32 + cq * 8), sp.hi);
-          tmem_st8(tmem_base + t_lane + 384u + (uint32_t)(j * 32 + cq * 8), sp.lo);
-          tmem_st_wait();
-          tc_fence_before();
-          __syncwarp();
-          if (lane == 0) mbar_arrive(&cs.a_ready[j]);
-        }
-        if (kTmemA) {
-          const uint32_t q = 34u * (uint32_t)it + (uint32_t)j, k = q / (uint32_t)kDgSlots;
-          const int slot = (int)(q % (uint32_t)kDgSlots);
-          uint8_t* st_hi = smem + kOffAct + (size_t)slot * 2 * kChunkBytes;
-          if (k > 0) mbar_wait(&cs.s_free[slot], (k - 1) & 1);
-          store16(sp, row, cq * kEpiCols, st_hi, st_hi + kChunkBytes);
-          if (!kStoreLsu) fence_proxy_async_smem();   // (LSU store warp: generic proxy on both sides)
-          __syncwarp();
-          if (lane == 0) mbar_arrive(&cs.g_ready[slot]);
-        } else {
-          const uint32_t n = 9u * (uint32_t)it;
-          if (n > 0) mbar_wait(&cs.s_free[j], (n - 1) & 1);
-          store16(sp, row, cq * kEpiCols, act_hi + (size_t)j * kChunkBytes, act_lo + (size_t)j * kChunkBytes);
-          fence_proxy_async_smem();
-          __syncwarp();
-          if (lane == 0) { mbar_arrive(&cs.a_ready[j]); mbar_arrive(&cs.g_ready[j]); }
-        }
+        tmem_st8(tmem_base + t_lane + 256u + (uint32_t)(j * 32 + cq * 8), sp.hi);
+        tmem_st8(tmem_base + t_lane + 384u + (uint32_t)(j * 32 + cq * 8), sp.lo);
+        tmem_st_wait();
+        tc_fence_before();
+        __syncwarp();
+        if (lane == 0) mbar_arrive(&cs.a_ready[j]);
+        const uint32_t qs = 34u * (uint32_t)it + (uint32_t)j, k = qs / (uint32_t)kDgSlots;
+        const int slot = (int)(qs % (uint32_t)kDgSlots);
+        uint8_t* st_hi = smem + kOffAct + (size_t)slot * 2 * kChunkBytes;
+        if (k > 0) mbar_wait(&cs.s_free[slot], (k - 1) & 1);
+        store16(sp, row, cq * kEpiCols, st_hi, st_hi + kChunkBytes);
+        fence_proxy_async_smem();
+        __syncwarp();
+        if (lane == 0) mbar_arrive(&cs.g_ready[slot]);
       }
 
       // ---------------- backward layers
       for (int bl = 0; bl < kNumBwdLayers; ++bl) {
-        const int buf = kTmemA ? 0 : (bl & 1);
         // ReLU mask of the forward activation this gradient flows into: feat (bl 0), h6 (bl 1), ... h0 (bl 7)
         long long tt = trace_tic();
         const uint2 mk = *p.img.mask_at(tile, bl == 0 ? 7 : 7 - bl, row, cq);
         const uint32_t masks[2] = {mk.x, mk.y};
         trace_toc(tr, 1, tt);
-        twait(tr, 0, &cs.d_full[buf], d_cnt[buf] & 1);
-        ++d_cnt[buf];
+        twait(tr, 0, &cs.d_full[0], d_cnt & 1);
+        ++d_cnt;
         tc_fence_after();
-        uint32_t vn[16];                            // accumulator columns of the NEXT block, loaded one block ahead
-        uint32_t va[kTmemA ? 4 : 1][16];            // kTmemA: this thread's whole share of the accumulator
-        if (kTmemA) {
+        uint32_t va[4][16];                         // this thread's whole share of the accumulator
+        long long tld = trace_tic();
 #pragma unroll
-          for (int j = 0; j < 4; ++j) tmem_ld16(tmem_base + t_lane + (uint32_t)(j * 64 + cq * kEpiCols), va[j]);
-          tmem_ld_wait();
-          tc_fence_before();
-          __syncwarp();
-          if (lane == 0) mbar_arrive(&cs.d_empty[0]);   // the (single) accumulator is free for the next layer's MMAs
-        } else {
-          tmem_ld16(tmem_base + t_lane + (uint32_t)(buf * 256 + cq * kEpiCols), vn);
-        }
+        for (int j = 0; j < 4; ++j) tmem_ld16(tmem_base + t_lane + (uint32_t)(j * 64 + cq * kEpiCols), va[j]);
+        tmem_ld_wait();
+        trace_toc(tr, 2, tld);
+        tc_fence_before();
+        __syncwarp();
+        if (lane == 0) mbar_arrive(&cs.d_empty[0]);   // the (single) accumulator is free for the next layer's MMAs
 #pragma unroll
         for (int j = 0; j < 4; ++j) {
-          uint32_t v[16];
           const int col0 = j * 64 + cq * kEpiCols;
-          long long tt2 = trace_tic();
-          if (kTmemA) {
-#pragma unroll
-            for (int i = 0; i < 16; ++i) v[i] = va[j][i];
-          } else {
-            tmem_ld_wait();
-#pragma unroll
-            for (int i = 0; i < 16; ++i) v[i] = vn[i];
-            if (j + 1 < 4) tmem_ld16(tmem_base + t_lane + (uint32_t)(buf * 256 + col0 + 64), vn);
-          }
-          trace_toc(tr, 2, tt2);
           float f[16];
           const uint32_t mask = (masks[j >> 1] >> (16 * (j & 1))) & 0xFFFFu;
 #pragma unroll
           for (int i = 0; i < 16; ++i) {
-            float g = __uint_as_float(v[i]);
+            float g = __uint_as_float(va[j][i]);
             if (bl == 1) g = fmaf(g_raw, s_w7r0[col0 + i], g);   // density row joins the feature gradient
             f[i] = ((mask >> i) & 1u) ? g : 0.f;
           }
-          const bool chain = bl != kNumBwdLayers - 1;   // G0 is only saved, nothing consumes it on-chip
           Split16 sp;
           split16<false>(f, sp);
-          if (kTmemA && chain) {
+          if (bl != kNumBwdLayers - 1) {   // G0 is only saved, nothing consumes it on-chip
             tmem_st8(tmem_base + t_lane + 256u + (uint32_t)(j * 32 + cq * 8), sp.hi);
             tmem_st8(tmem_base + t_lane + 384u + (uint32_t)(j * 32 + cq * 8), sp.lo);
             tmem_st_wait();
@@ -1381,33 +1202,15 @@ __global__ void __launch_bounds__(kThreads, 1) tc_mlp_dgrad_kernel(const BwdPara
             if (lane == 0) mbar_arrive(&cs.a_ready[j]);
           }
           long long tt3 = trace_tic();
-          if (kTmemA) {
-            const uint32_t q = 34u * (uint32_t)it + 2u + 4u * (uint32_t)bl + (uint32_t)j, k = q / (uint32_t)kDgSlots;
-            const int slot = (int)(q % (uint32_t)kDgSlots);
-            uint8_t* st_hi = smem + kOffAct + (size_t)slot * 2 * kChunkBytes;
-            if (k > 0) mbar_wait(&cs.s_free[slot], (k - 1) & 1);
-            trace_toc(tr, 3, tt3);
-            store16(sp, row, cq * kEpiCols, st_hi, st_hi + kChunkBytes);
-            if (!kStoreLsu) fence_proxy_async_smem();
-            __syncwarp();
-            if (lane == 0) mbar_arrive(&cs.g_ready[slot]);
-          } else {
-            const uint32_t n = j < 2 ? 9u * (uint32_t)it + (uint32_t)bl + 1u : 8u * (uint32_t)it + (uint32_t)bl;
-            if (n > 0) mbar_wait(&cs.s_free[j], (n - 1) & 1);
-            trace_toc(tr, 3, tt3);
-            store16(sp, row, cq * kEpiCols, act_hi + (size_t)j * kChunkBytes, act_lo + (size_t)j * kChunkBytes);
-            fence_proxy_async_smem();
-            __syncwarp();
-            if (lane == 0) {
-              if (chain) mbar_arrive(&cs.a_ready[j]);
-              mbar_arrive(&cs.g_ready[j]);
-            }
-          }
-        }
-        if (!kTmemA) {
-          tc_fence_before();
+          const uint32_t qs = 34u * (uint32_t)it + 2u + 4u * (uint32_t)bl + (uint32_t)j, k = qs / (uint32_t)kDgSlots;
+          const int slot = (int)(qs % (uint32_t)kDgSlots);
+          uint8_t* st_hi = smem + kOffAct + (size_t)slot * 2 * kChunkBytes;
+          if (k > 0) mbar_wait(&cs.s_free[slot], (k - 1) & 1);
+          trace_toc(tr, 3, tt3);
+          store16(sp, row, cq * kEpiCols, st_hi, st_hi + kChunkBytes);
+          fence_proxy_async_smem();
           __syncwarp();
-          if (lane == 0) mbar_arrive(&cs.d_empty[buf]);
+          if (lane == 0) mbar_arrive(&cs.g_ready[slot]);
         }
       }
     }
@@ -1443,8 +1246,6 @@ struct WgradJob {
                          // not read at all (the bias gradients become column sums of G_hi)
 };
 constexpr int kMaxWgradJobs = 160;
-constexpr int kBwdSplitDefault = 1;     // sub-chunks of the backward pipeline (dgrad(k + 1) beside wgrad(k)); 1 = off
-constexpr int kBwdNdDefault = 88;       // SMs of the dgrad chain while a weight-gradient kernel runs beside it
 struct WgradJobs { WgradJob j[kMaxWgradJobs]; };   // passed by value (kernel parameter): no host->device copy per step
 constexpr int kWgStages = 3;                // three passes: 3 stages of 64 KB; one pass (hi halves only): 6 stages of 32 KB, so
 constexpr int kWgMaxStages = 6;             // that the same number of bytes is in flight per SM (the kernel is HBM-latency bound)
@@ -1622,7 +1423,7 @@ __device__ __forceinline__ float img_value(const Images& img, int t, long long m
   return __uint_as_float((uint32_t)hi << 16) + __uint_as_float((uint32_t)lo << 16);
 }
 
-// One launch for every row-reduction over the saved images (bias gradients and the two narrow layers):
+// One row-reduction over the saved images per launch (bias gradients and the two narrow layers):
 //   mode 0:  out[f]            += sum_m img[m][f]                                   (colsum -> bias grads)
 //   mode 1/3: out[c*ldo + f]   += sum_m g[m*gs + c] * img[m][f], out_bias[c] += sum_m g[m*gs + c]
 // Block = 256 threads = 8 row groups x 32 sixteen-byte chunks (8 features each); a block owns a few row
@@ -1638,13 +1439,10 @@ struct ReduceJob {
   int parts;           // 2: image = hi + lo halves; 1: hi half only (the lo half was not written: SPARF_ENGINE_TC_3X_W1)
 };
 
-struct ReduceJobs { ReduceJob j[16]; };
-
 template <int NC>   // NC = 0 (column sums) | 1 | 3 narrow outputs: sizes the accumulators (registers -> blocks per SM)
-__global__ void __launch_bounds__(256) image_reduce_kernel(const __grid_constant__ ReduceJobs jobs, Images img, long long M,
+__global__ void __launch_bounds__(256) image_reduce_kernel(const __grid_constant__ ReduceJob job, Images img, long long M,
                                                            int ntiles, int tiles_per_block) {
   __shared__ float red[8][32][25];
-  const ReduceJob& job = jobs.j[blockIdx.y];
   const int tid = threadIdx.x, c16 = tid & 31, rg = tid >> 5;
   const int fb = c16 >> 3, c = c16 & 7;
   const bool active = fb < job.nblk;
@@ -1978,7 +1776,6 @@ bool tc_supports(const SparfMLP* mlp) {
          mlp->L_xyz == kL && mlp->L_view == kLv;
 }
 
-bool tc_backward_available() { return true; }
 static int tape_tiles(int R, int S);
 static size_t tape_off_denc(int R, int S);
 static size_t tape_off_packed_b(int R, int S);
@@ -2019,8 +1816,6 @@ struct BwdCarve {
   uint8_t *packed_f, *packed_b, *images_f, *images_b;
   float *raybias, *denc, *sigma, *rgb, *g_raw, *g_pre, *rayS, *gdenc;
   uint8_t* packed_e;
-  WgradJob* jobs;
-  ReduceJob* rjobs;
   size_t total;
 };
 
@@ -2033,15 +1828,30 @@ static BwdCarve bwd_carve(void* ws, int nr, int S, bool with_fwd_images) {
   uint8_t* b = reinterpret_cast<uint8_t*>(ws);
   size_t o_pf = take((size_t)kChunksPerTile * kChunkBytes), o_pb = take((size_t)kBwdChunksPerTile * kChunkBytes);
   size_t o_rb = take((size_t)nr * kHW * 4), o_de = take((size_t)nr * 32 * 4), o_si = take(Mc * 4), o_rg = take(Mc * 12);
-  size_t o_gr = take(Mc * 4), o_gp = take(Mc * 16), o_rs = take((size_t)nr * kHW * 4), o_jb = take(256 * sizeof(WgradJob));
-  size_t o_rj = take(16 * sizeof(ReduceJob));
+  size_t o_gr = take(Mc * 4), o_gp = take(Mc * 16), o_rs = take((size_t)nr * kHW * 4);
   size_t o_gd = take((size_t)nr * 32 * 4), o_pe = take(kEgWBytes);
   size_t o_ib = take(bwd_images_bytes(ntiles));
   size_t o_if = take(with_fwd_images ? fwd_images_bytes(ntiles) : 0);
   c.packed_f = b + o_pf; c.packed_b = b + o_pb; c.raybias = (float*)(b + o_rb); c.denc = (float*)(b + o_de);
   c.sigma = (float*)(b + o_si); c.rgb = (float*)(b + o_rg); c.g_raw = (float*)(b + o_gr); c.g_pre = (float*)(b + o_gp);
-  c.rayS = (float*)(b + o_rs); c.jobs = (WgradJob*)(b + o_jb); c.rjobs = (ReduceJob*)(b + o_rj); c.gdenc = (float*)(b + o_gd); c.packed_e = b + o_pe; c.images_b = b + o_ib; c.images_f = with_fwd_images ? b + o_if : nullptr;
+  c.rayS = (float*)(b + o_rs); c.gdenc = (float*)(b + o_gd); c.packed_e = b + o_pe; c.images_b = b + o_ib; c.images_f = with_fwd_images ? b + o_if : nullptr;
   c.total = o + 1024;
+  return c;
+}
+
+// forward workspace (inference and taped forward): packed forward weight stream | raybias [R,128]
+struct FwdCarve {
+  uint8_t* packed;
+  float* raybias;
+  size_t total;
+};
+
+static FwdCarve fwd_carve(void* ws, int R) {
+  const size_t o_rb = align_up((size_t)kChunksPerTile * kChunkBytes, 256);
+  FwdCarve c;
+  c.packed = reinterpret_cast<uint8_t*>(ws);
+  c.raybias = reinterpret_cast<float*>(c.packed + o_rb);
+  c.total = o_rb + align_up((size_t)R * kHW * sizeof(float), 256) + 256;
   return c;
 }
 
@@ -2050,7 +1860,7 @@ size_t tc_workspace_bytes(const SparfMLP* mlp, int R, int S, int backward, int e
     int nr = std::min(R, bwd_chunk_rays(S));
     return bwd_carve(nullptr, nr, S, backward != 2).total;
   }
-  return align_up((size_t)16 * kChunksPerTile * kChunkBytes, 256) + align_up((size_t)R * kHW * sizeof(float), 256) + 256;
+  return fwd_carve(nullptr, R).total;
 }
 
 static void fill_pack_params(const SparfMLP* mlp, PackParams& pp, uint8_t* dst) {
@@ -2060,23 +1870,9 @@ static void fill_pack_params(const SparfMLP* mlp, PackParams& pp, uint8_t* dst) 
   pp.order = 0;
 }
 
-static int weight_copies() {
-  static int v = -1;
-  if (v < 0) {
-    const char* e = getenv("SPARF_TC_WCOPIES");
-    v = e ? std::max(1, std::min(16, atoi(e))) : 1;
-  }
-  return v;
-}
-
-// which forward kernel serves a call: FWD_TMEM = the A operand in tensor memory (fp16 3-pass: every default call;
-// SPARF_TC_TMEMA=0 disables it), FWD_SMEM = operands in shared memory (single-pass engine, bf16 recompute forward)
-enum { FWD_SMEM = 0, FWD_TMEM = 2 };
-static int fwd_variant(bool f16, int passes, bool save, int num_tiles) {
-  static const bool tmem_ok = !(getenv("SPARF_TC_TMEMA") && getenv("SPARF_TC_TMEMA")[0] == '0');
-  (void)save; (void)num_tiles;
-  return (tmem_ok && f16 && passes == 3) ? FWD_TMEM : FWD_SMEM;
-}
+// which forward kernel serves a call: the A operand in tensor memory for fp16 3-pass calls (every default call), operands
+// in shared memory otherwise (single-pass engine, bf16 recompute forward).  The weight packing order follows it.
+static bool fwd_tmem(bool f16, int passes) { return f16 && passes == 3; }
 
 #ifdef SPARF_TC_TRACE
 static void trace_dump(const char* what) {
@@ -2110,7 +1906,7 @@ static void trace_dump(const char* what) {
 
 static int launch_forward(const SparfMLP* mlp, bool f16, int passes, int nr, int S, const float* origins, const float* dirs,
                           const float* t, const float* noise, float* sigma, float* rgb, const uint8_t* packed,
-                          const float* raybias, const Images* img, cudaStream_t st, int ncopies = 1, int save_mode = 1) {
+                          const float* raybias, const Images* img, cudaStream_t st, int save_mode = 1) {
   FwdParams p;
   p.packed = packed;
   p.raybias = raybias;
@@ -2125,7 +1921,6 @@ static int launch_forward(const SparfMLP* mlp, bool f16, int passes, int nr, int
   p.S = S;
   p.num_tiles = (int)((p.M + kTileM - 1) / kTileM);
   p.passes = passes;
-  p.ncopies = ncopies;
   p.save = img != nullptr ? save_mode : 0;
   if (img) p.img = *img; else { for (int i = 0; i < T_COUNT; ++i) p.img.ptr[i] = nullptr; }
   static bool attr_set_dev[64] = {};
@@ -2137,18 +1932,17 @@ static int launch_forward(const SparfMLP* mlp, bool f16, int passes, int nr, int
     SPARF_CHECK_CUDA(cudaFuncSetAttribute(tc_mlp_fwd_kernel<true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemBytes + 1024));
     SPARF_CHECK_CUDA(cudaFuncSetAttribute(tc_mlp_fwd_kernel<true, true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemBytes + 1024));
     SPARF_CHECK_CUDA(cudaFuncSetAttribute(tc_mlp_fwd_kernel<false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemBytes + 1024));
-    SPARF_CHECK_CUDA(cudaFuncSetAttribute(tc_mlp_dgrad_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemBytes + 1024));
-    SPARF_CHECK_CUDA(cudaFuncSetAttribute(tc_mlp_dgrad_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemBytes + 1024));
+    SPARF_CHECK_CUDA(cudaFuncSetAttribute(tc_mlp_dgrad_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemBytes + 1024));
     SPARF_CHECK_CUDA(cudaFuncSetAttribute(tc_mlp_wgrad_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kWgSmem + 1024));
     SPARF_CHECK_CUDA(cudaFuncSetAttribute(tc_mlp_encgrad_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kEgSmem + 1024));
     attr_set = true;
   }
-  const int variant = fwd_variant(f16, passes, p.save != 0, p.num_tiles);
-  if (variant != FWD_TMEM && p.save == 2) p.save = 1;     // the shared-memory-operand kernels always write both halves
-  if (variant == FWD_TMEM && p.save == 2) {
+  const bool tmem = fwd_tmem(f16, passes);
+  if (!tmem && p.save == 2) p.save = 1;     // the shared-memory-operand kernels always write both halves
+  if (tmem && p.save == 2) {
     tc_mlp_fwd_kernel<true, true, true><<<std::min(p.num_tiles, num_sms()), kThreads, kSmemBytes + 1024, st>>>(p);
     TRACE_DUMP("forward (hi-only tape, A in TMEM)");
-  } else if (variant == FWD_TMEM) {
+  } else if (tmem) {
     tc_mlp_fwd_kernel<true, true><<<std::min(p.num_tiles, num_sms()), kThreads, kSmemBytes + 1024, st>>>(p);
     TRACE_DUMP(p.save ? "forward (tape, A in TMEM)" : "forward f16 (A in TMEM)");
   } else {
@@ -2174,19 +1968,17 @@ int tc_mlp_forward(const SparfMLP* mlp, int engine, int R, int S, const float* o
     set_error("tc_mlp_forward: workspace %zu < %zu bytes", workspace_bytes, tc_workspace_bytes(mlp, R, S, 0, engine));
     return SPARF_ERR_WORKSPACE;
   }
-  uint8_t* packed = reinterpret_cast<uint8_t*>(workspace);
-  float* raybias = reinterpret_cast<float*>(packed + align_up((size_t)16 * kChunksPerTile * kChunkBytes, 256));
+  const FwdCarve ws = fwd_carve(workspace, R);
+  const int passes = engine == SPARF_ENGINE_TC_1X ? 1 : 3;
   PackParams pp;
-  fill_pack_params(mlp, pp, packed);
-  const int passes_ = engine == SPARF_ENGINE_TC_1X ? 1 : 3;
-  pp.order = fwd_variant(true, passes_, false, (int)(((long long)R * S + kTileM - 1) / kTileM)) == FWD_TMEM ? 1 : 0;
-  pack_weights_kernel<true><<<dim3(kChunksPerTile, weight_copies()), 1024, 0, st>>>(pp);   // one element group per thread
+  fill_pack_params(mlp, pp, ws.packed);
+  pp.order = fwd_tmem(true, passes) ? 1 : 0;
+  pack_weights_kernel<true><<<kChunksPerTile, 1024, 0, st>>>(pp);   // one element group per thread
   SPARF_CHECK_LAUNCH("pack_weights_kernel");
   C2F c2f{mlp->use_c2f, mlp->c2f_start, mlp->c2f_range, mlp->progress};
-  raybias_kernel<<<ceil_div(R, 4), 512, 0, st>>>(R, dirs, mlp->head_w[0], mlp->head_b[0], c2f, raybias, nullptr);
+  raybias_kernel<<<ceil_div(R, 4), 512, 0, st>>>(R, dirs, mlp->head_w[0], mlp->head_b[0], c2f, ws.raybias, nullptr);
   SPARF_CHECK_LAUNCH("raybias_kernel");
-  return launch_forward(mlp, true, engine == SPARF_ENGINE_TC_1X ? 1 : 3, R, S, origins, dirs, t, noise, sigma, rgb, packed,
-                        raybias, nullptr, st, weight_copies());
+  return launch_forward(mlp, true, passes, R, S, origins, dirs, t, noise, sigma, rgb, ws.packed, ws.raybias, nullptr, st);
 }
 
 // Fork / join onto a library-owned side stream (one per device, created on first use): the CUDA-core leftovers of the
@@ -2194,53 +1986,32 @@ int tc_mlp_forward(const SparfMLP* mlp, int engine, int R, int S, const float* o
 // they run BESIDE the HBM-bound weight-gradient kernel instead of after it (its CTAs leave ~30 KB of shared memory and
 // most thread slots of every SM free).  Event record / wait pairs make the pattern capturable into a CUDA graph.
 struct SideStream {
+  bool ready = false;
   cudaStream_t stream = nullptr;
   cudaStream_t stream2 = nullptr, stream3 = nullptr;   // backward leftovers: three independent chains beside the wgrad kernel
   cudaEvent_t join2 = nullptr, join3 = nullptr, rayhead = nullptr;
   cudaEvent_t fork = nullptr, join = nullptr;
   cudaEvent_t raybias = nullptr, packed = nullptr;   // taped forward: raybias ready / backward weight streams packed
-  cudaEvent_t sub[8] = {};                           // backward: dgrad of sub-chunk k finished
 };
+// nullptr (with the error text set) if the streams or events cannot be created
 static SideStream* side_stream() {
   static SideStream table[64];
   int dev = 0;
   cudaGetDevice(&dev);
   SideStream& s = table[dev & 63];
-  if (!s.stream) {
-    if (cudaStreamCreateWithFlags(&s.stream, cudaStreamNonBlocking) != cudaSuccess) return nullptr;
-    if (cudaStreamCreateWithFlags(&s.stream2, cudaStreamNonBlocking) != cudaSuccess ||
-        cudaStreamCreateWithFlags(&s.stream3, cudaStreamNonBlocking) != cudaSuccess) { s.stream = nullptr; return nullptr; }
-    cudaEventCreateWithFlags(&s.join2, cudaEventDisableTiming);
-    cudaEventCreateWithFlags(&s.join3, cudaEventDisableTiming);
-    cudaEventCreateWithFlags(&s.rayhead, cudaEventDisableTiming);
-    cudaEventCreateWithFlags(&s.fork, cudaEventDisableTiming);
-    cudaEventCreateWithFlags(&s.join, cudaEventDisableTiming);
-    cudaEventCreateWithFlags(&s.raybias, cudaEventDisableTiming);
-    cudaEventCreateWithFlags(&s.packed, cudaEventDisableTiming);
-    for (auto& e : s.sub) cudaEventCreateWithFlags(&e, cudaEventDisableTiming);
+  if (!s.ready) {
+    cudaError_t e = cudaSuccess;
+    for (cudaStream_t* p : {&s.stream, &s.stream2, &s.stream3})
+      if (e == cudaSuccess && !*p) e = cudaStreamCreateWithFlags(p, cudaStreamNonBlocking);
+    for (cudaEvent_t* p : {&s.join2, &s.join3, &s.rayhead, &s.fork, &s.join, &s.raybias, &s.packed})
+      if (e == cudaSuccess && !*p) e = cudaEventCreateWithFlags(p, cudaEventDisableTiming);
+    if (e != cudaSuccess) {
+      set_error("tcgen05 engine: cannot create its side streams: %s", cudaGetErrorString(e));
+      return nullptr;
+    }
+    s.ready = true;
   }
   return &s;
-}
-// Backward pipelining (SPARF_TC_BWD_SPLIT = n sub-chunks, SPARF_TC_BWD_ND = SMs given to the dgrad chain while a
-// weight-gradient kernel runs beside it; 0 / 1 = off): the dgrad chain is tensor-bound, the weight-gradient pass
-// HBM-bound, so dgrad(k + 1) and wgrad(k) run concurrently on disjoint SM sets (grid sizes; one CTA per SM either way).
-static int bwd_split_env(const char* name, int dflt) {
-  const char* e = getenv(name);
-  return e ? atoi(e) : dflt;
-}
-__host__ __device__ inline void images_advance(Images& img, int tile0) {
-  for (int t = 0; t < T_COUNT; ++t)
-    if (img.ptr[t]) img.ptr[t] += (size_t)tile0 * tensor_nblk(t) * 2 * kChunkBytes;
-  if (img.mask) img.mask += (size_t)tile0 * kMaskTileBytes;
-}
-
-static bool overlap_small_kernels() {
-  static int v = -1;
-  if (v < 0) {
-    const char* e = getenv("SPARF_TC_OVERLAP");     // 0: everything on the caller's stream (debugging / A-B timing)
-    v = (e && e[0] == '0') ? 0 : 1;
-  }
-  return v == 1;
 }
 
 // Training forward: same fp16-split arithmetic and outputs as tc_mlp_forward, plus the tape for the backward.
@@ -2258,48 +2029,42 @@ int tc_mlp_forward_tape(const SparfMLP* mlp, int engine, int R, int S, const flo
     set_error("tc_mlp_forward_tape: workspace %zu < %zu bytes", workspace_bytes, tc_workspace_bytes(mlp, R, S, 0, engine));
     return SPARF_ERR_WORKSPACE;
   }
-  uint8_t* packed = reinterpret_cast<uint8_t*>(workspace);
-  float* raybias = reinterpret_cast<float*>(packed + align_up((size_t)kChunksPerTile * kChunkBytes, 256));
+  const FwdCarve ws = fwd_carve(workspace, R);
   const int ntiles = tape_tiles(R, S);
   uint8_t* tp = reinterpret_cast<uint8_t*>(tape);
   float* denc = reinterpret_cast<float*>(tp + tape_off_denc(R, S));
   C2F c2f{mlp->use_c2f, mlp->c2f_start, mlp->c2f_range, mlp->progress};
   // side stream: the per-ray colour-head bias (needed by the forward kernel) and the two weight streams of the
   // BACKWARD (needed only by sparf_mlp_backward_tape) run beside the forward packing / kernel
-  SideStream* side = overlap_small_kernels() ? side_stream() : nullptr;
-  cudaStream_t sd = st;
-  if (side) {
-    SPARF_CHECK_CUDA(cudaEventRecord(side->fork, st));
-    SPARF_CHECK_CUDA(cudaStreamWaitEvent(side->stream, side->fork, 0));
-    sd = side->stream;
-  }
-  raybias_kernel<<<ceil_div(R, 4), 512, 0, sd>>>(R, dirs, mlp->head_w[0], mlp->head_b[0], c2f, raybias, denc);
+  SideStream* side = side_stream();
+  if (!side) return SPARF_ERR_CUDA;
+  SPARF_CHECK_CUDA(cudaEventRecord(side->fork, st));
+  SPARF_CHECK_CUDA(cudaStreamWaitEvent(side->stream, side->fork, 0));
+  raybias_kernel<<<ceil_div(R, 4), 512, 0, side->stream>>>(R, dirs, mlp->head_w[0], mlp->head_b[0], c2f, ws.raybias, denc);
   SPARF_CHECK_LAUNCH("raybias_kernel");
-  if (side) SPARF_CHECK_CUDA(cudaEventRecord(side->raybias, side->stream));
+  SPARF_CHECK_CUDA(cudaEventRecord(side->raybias, side->stream));
   PackParams pp;
-  fill_pack_params(mlp, pp, packed);
-  pp.order = fwd_variant(true, 3, true, ntiles) == FWD_TMEM ? 1 : 0;
+  fill_pack_params(mlp, pp, ws.packed);
+  pp.order = fwd_tmem(true, 3) ? 1 : 0;
   pack_weights_kernel<true><<<kChunksPerTile, 1024, 0, st>>>(pp);   // on the forward's critical path: one element group
                                                                       // per thread (13 -> ~6 us)
   SPARF_CHECK_LAUNCH("pack_weights_kernel");
   PackParams pb;
   fill_pack_params(mlp, pb, tp + tape_off_packed_b(R, S));
-  pack_weights_bwd_kernel<<<kBwdChunksPerTile, 256, 0, sd>>>(pb);
+  pack_weights_bwd_kernel<<<kBwdChunksPerTile, 256, 0, side->stream>>>(pb);
   SPARF_CHECK_LAUNCH("pack_weights_bwd_kernel");
-  pack_weights_enc_kernel<<<16, 256, 0, sd>>>(mlp->trunk_w[4], mlp->trunk_w[0], tp + tape_off_packed_e(R, S));
+  pack_weights_enc_kernel<<<16, 256, 0, side->stream>>>(mlp->trunk_w[4], mlp->trunk_w[0], tp + tape_off_packed_e(R, S));
   SPARF_CHECK_LAUNCH("pack_weights_enc_kernel");
-  if (side) {
-    SPARF_CHECK_CUDA(cudaEventRecord(side->packed, side->stream));
-    SPARF_CHECK_CUDA(cudaStreamWaitEvent(st, side->raybias, 0));
-  }
+  SPARF_CHECK_CUDA(cudaEventRecord(side->packed, side->stream));
+  SPARF_CHECK_CUDA(cudaStreamWaitEvent(st, side->raybias, 0));
   Images img;
   images_assign(img, ntiles, tp, nullptr);
   // TC_3X_W1: the weight gradients will take the hi halves only, so only those are written (the tape keeps its layout)
-  rc = launch_forward(mlp, true, 3, R, S, origins, dirs, t, noise, sigma, rgb, packed, raybias, &img, st, 1,
+  rc = launch_forward(mlp, true, 3, R, S, origins, dirs, t, noise, sigma, rgb, ws.packed, ws.raybias, &img, st,
                       engine == SPARF_ENGINE_TC_3X_W1 ? 2 : 1);
   // join: whatever follows on the caller's stream (the backward, or a reuse of the tape's memory) is ordered after the
   // side-stream packing, which has long finished by the time the forward kernel ends
-  if (side && rc == SPARF_OK) SPARF_CHECK_CUDA(cudaStreamWaitEvent(st, side->packed, 0));
+  if (rc == SPARF_OK) SPARF_CHECK_CUDA(cudaStreamWaitEvent(st, side->packed, 0));
   return rc;
 }
 
@@ -2360,6 +2125,8 @@ static int tc_mlp_backward_impl(const SparfMLP* mlp, int engine, int R, int S, c
     set_error("tc_mlp_backward: workspace %zu < %zu bytes", workspace_bytes, tc_workspace_bytes(mlp, R, S, tape ? 2 : 1, engine));
     return SPARF_ERR_WORKSPACE;
   }
+  SideStream* side = side_stream();
+  if (!side) return SPARF_ERR_CUDA;
   const int nrc = std::min(R, bwd_chunk_rays(S));
   const C2F c2f{mlp->use_c2f, mlp->c2f_start, mlp->c2f_range, mlp->progress};
   for (int r0 = 0; r0 < R; r0 += nrc) {
@@ -2412,119 +2179,67 @@ static int tc_mlp_backward_impl(const SparfMLP* mlp, int engine, int R, int S, c
     bp.g_raw = c.g_raw; bp.g_pre = c.g_pre;
     bp.w7 = mlp->trunk_w[7]; bp.w9 = mlp->head_w[1];
     bp.M = Mc; bp.num_tiles = ntiles; bp.img = img;
-    static const bool tmem_a = !(getenv("SPARF_TC_TMEMA") && getenv("SPARF_TC_TMEMA")[0] == '0');
-    static const bool overlap_bwd = !(getenv("SPARF_TC_OVERLAP_BWD") && getenv("SPARF_TC_OVERLAP_BWD")[0] == '0');
-    SideStream* side = (overlap_small_kernels() && overlap_bwd) ? side_stream() : nullptr;
-    // sub-chunk pipeline only with the TMEM-operand chain kernel and when every sub-chunk still fills the GPU
-    int nsplit = (side && tmem_a) ? std::min(8, std::max(1, bwd_split_env("SPARF_TC_BWD_SPLIT", kBwdSplitDefault))) : 1;
-    while (nsplit > 1 && ntiles / nsplit < num_sms()) --nsplit;
-    const int nd_sms = std::max(16, std::min(num_sms() - 16, bwd_split_env("SPARF_TC_BWD_ND", kBwdNdDefault)));
+    // A operand in tensor memory (shared-memory operands measured 360 vs 294 us, profiles/r02_notes.md)
+    tc_mlp_dgrad_kernel<<<std::min(ntiles, num_sms()), kThreads, kSmemBytes + 1024, st>>>(bp);
+    TRACE_DUMP("dgrad");
+    SPARF_CHECK_LAUNCH("tc_mlp_dgrad_kernel");
 
-    // 3. (helper) weight-gradient job table = (layer, slab of row tiles) over tiles [t_lo, t_hi), ~`ctas` CTAs, one per SM
-    auto wgrad_launch = [&](int t_lo, int t_hi, int ctas, cudaStream_t ws) -> int {
-      WgradJobs jobs_tab;
-      WgradJob* jobs = jobs_tab.j;
-      int nj = 0;
-      const int nt = t_hi - t_lo;
-      auto add_jobs = [&](int tg, int tx, int mblk, int nblk, float* dW, int ldw, int col0, int enc, int slabs, float* colsum) {
-        slabs = std::max(1, std::min(slabs, nt));
-        for (int sl = 0; sl < slabs; ++sl) {
-          WgradJob j;
-          j.t_g = tg; j.t_x = tx; j.mblk = mblk; j.nblk = nblk;
-          j.tile_begin = t_lo + (int)((long long)nt * sl / slabs);
-          j.tile_end = t_lo + (int)((long long)nt * (sl + 1) / slabs);
-          j.dW = dW; j.ldw = ldw; j.col0 = col0; j.enc_cols = enc; j.colsum = colsum;
-          j.passes = wg_passes;
-          jobs[nj++] = j;
-        }
-      };
-      // One CTA per SM in a single wave.  A stage (32 rows of one tile) costs about the same ~2.4k clocks whatever its
-      // width (it is bound by the latency of the 3-deep HBM pipeline, profiles/r01_ncu_chain.md), so the slabs equalise
-      // the number of stages per CTA rather than bytes: 10 job types x ~14.8 slabs = 147 CTAs on a whole GPU.
-      int slabs[10];      // 8 wide job types, then the two encoder-block types
-      const int s_lo = std::max(1, ctas / 10), extra = std::max(0, std::min(8, ctas - 10 * s_lo));
-      for (int i = 0; i < 10; ++i) slabs[i] = s_lo + (i < extra ? 1 : 0);
-      add_jobs(T_GHID, T_FEAT, 2, 4, grad->head_w[0], kW + kEv, 0, 0, slabs[7], grad->head_b[0]);     // head 0, feature part
-      add_jobs(T_G7F, T_H0 + 6, 4, 4, grad->trunk_w[7] + kW, kW, 0, 0, slabs[0], grad->trunk_b[7] + 1);  // trunk 7 rows 1..256
-      for (int l = 6; l >= 1; --l)
-        add_jobs(t_g(l), T_H0 + (l - 1), 4, 4, grad->trunk_w[l], l == 4 ? kW + 63 : kW, 0, 0, slabs[7 - l], grad->trunk_b[l]);
-      add_jobs(t_g(4), T_ENC, 4, 1, grad->trunk_w[4], kW + 63, kW, 1, slabs[8], nullptr);             // skip part of layer 4
-      add_jobs(t_g(0), T_ENC, 4, 1, grad->trunk_w[0], 63, 0, 1, slabs[9], grad->trunk_b[0]);          // layer 0 (+ its bias)
-      tc_mlp_wgrad_kernel<<<nj, 192, kWgSmem + 1024, ws>>>(jobs_tab, img);
-      SPARF_CHECK_LAUNCH("tc_mlp_wgrad_kernel");
-      return SPARF_OK;
-    };
-
-    // streams of the CUDA-core leftovers (steps 4, 5): up to three independent chains, so that together they are shorter
-    // than the weight-gradient kernel they run beside (each is slowed down several-fold while it shares the GPU with it)
-    cudaStream_t sd = st, sd2 = st, sd3 = st;
-    if (nsplit <= 1) {
-      // A operand in tensor memory (default; SPARF_TC_TMEMA=0 selects the shared-memory-operand kernel): 294 vs 360 us
-      if (tmem_a) tc_mlp_dgrad_kernel<true><<<std::min(ntiles, num_sms()), kThreads, kSmemBytes + 1024, st>>>(bp);
-      else tc_mlp_dgrad_kernel<false><<<std::min(ntiles, num_sms()), kThreads, kSmemBytes + 1024, st>>>(bp);
-      TRACE_DUMP("dgrad");
-      SPARF_CHECK_LAUNCH("tc_mlp_dgrad_kernel");
-    }
-    if (nsplit <= 1) {
-      // fork: the leftovers run on the side stream beside the weight-gradient kernel (or everything on `st`)
-      if (side) {
-        SPARF_CHECK_CUDA(cudaEventRecord(side->fork, st));
-        SPARF_CHECK_CUDA(cudaStreamWaitEvent(side->stream, side->fork, 0));
-        sd = sd2 = sd3 = side->stream;
-        // with ray gradients the leftovers (reductions + ray-gradient GEMM + view-direction chain) are longer than the
-        // weight-gradient kernel when serialised: three chains (c3: 4.46 -> 4.39 ms); without them one chain is enough
-        // and measured marginally faster (c2: 1.335 vs 1.345 ms)
-        // (the single-pass weight-gradient kernel is short enough that the serial chain outlasts it even without them)
-        if (d_origins != nullptr || d_dirs != nullptr || wg_passes == 1) {
-          SPARF_CHECK_CUDA(cudaStreamWaitEvent(side->stream2, side->fork, 0));
-          SPARF_CHECK_CUDA(cudaStreamWaitEvent(side->stream3, side->fork, 0));
-          sd2 = side->stream2; sd3 = side->stream3;
-        }
-      }
-      rc = wgrad_launch(0, ntiles, num_sms() - 1, st);
-      if (rc) return rc;
-    } else {
-      // pipeline: dgrad(0) on every SM, then dgrad(k) on nd_sms SMs beside wgrad(k - 1) on the others (side stream),
-      // the last wgrad on every SM beside the leftovers (caller's stream)
-      for (int k = 0; k < nsplit; ++k) {
-        const int t_lo = (int)((long long)ntiles * k / nsplit), t_hi = (int)((long long)ntiles * (k + 1) / nsplit);
-        BwdParams bk = bp;
-        const long long m_off = (long long)t_lo * kTileM;
-        bk.d_sigma += m_off; bk.d_rgb += m_off * 3; bk.sigma += m_off; bk.rgb += m_off * 3;
-        bk.g_raw += m_off; bk.g_pre += m_off * 4;
-        bk.num_tiles = t_hi - t_lo;
-        bk.M = std::min<long long>(Mc - m_off, (long long)bk.num_tiles * kTileM);
-        images_advance(bk.img, t_lo);
-        const int grid = std::min(bk.num_tiles, k == 0 ? num_sms() : nd_sms);
-        tc_mlp_dgrad_kernel<true><<<grid, kThreads, kSmemBytes + 1024, st>>>(bk);
-        SPARF_CHECK_LAUNCH("tc_mlp_dgrad_kernel");
-        SPARF_CHECK_CUDA(cudaEventRecord(side->sub[k], st));
-        SPARF_CHECK_CUDA(cudaStreamWaitEvent(side->stream, side->sub[k], 0));
-        rc = wgrad_launch(t_lo, t_hi, k + 1 < nsplit ? num_sms() - nd_sms : num_sms() - 1, side->stream);
-        if (rc) return rc;
-      }
+    // fork: the CUDA-core leftovers (steps 4, 5) run on the side streams beside the weight-gradient kernel
+    SPARF_CHECK_CUDA(cudaEventRecord(side->fork, st));
+    SPARF_CHECK_CUDA(cudaStreamWaitEvent(side->stream, side->fork, 0));
+    cudaStream_t sd = side->stream, sd2 = side->stream, sd3 = side->stream;
+    // Up to three independent chains, so that together they are shorter than the weight-gradient kernel they run beside
+    // (each is slowed down several-fold while it shares the GPU with it).  With ray gradients the leftovers
+    // (reductions + ray-gradient GEMM + view-direction chain) are longer than the weight-gradient kernel when serialised:
+    // three chains (c3: 4.46 -> 4.39 ms); without them one chain is enough and measured marginally faster (c2: 1.335 vs
+    // 1.345 ms).  (The single-pass weight-gradient kernel is short enough that the serial chain outlasts it even without
+    // them.)
+    if (d_origins != nullptr || d_dirs != nullptr || wg_passes == 1) {
+      SPARF_CHECK_CUDA(cudaStreamWaitEvent(side->stream2, side->fork, 0));
+      SPARF_CHECK_CUDA(cudaStreamWaitEvent(side->stream3, side->fork, 0));
+      sd2 = side->stream2; sd3 = side->stream3;
     }
 
-    // 4. CUDA-core leftovers: biases, density row, 128->3 head, view-direction columns
-    ReduceJobs rj_tab;
-    ReduceJob* rj = rj_tab.j;
-    int nrj = 0;
-    auto add_red = [&](int t, int nblk, int nc, const float* g, int gs, float* out, int ldo, float* ob) {
-      ReduceJob j; j.t = t; j.nblk = nblk; j.nc = nc; j.g = g; j.gs = gs; j.out = out; j.ldo = ldo; j.out_bias = ob;
-      j.parts = (tape && wg_passes == 1) ? 1 : 2;     // forward images of a TC_3X_W1 tape hold their hi halves only
-      rj[nrj++] = j;
+    // 3. weight-gradient jobs = (layer, slab of row tiles), one CTA on every SM but one, in a single wave.  A stage (32 rows of one tile) costs about the same ~2.4k clocks whatever its width (it is bound by
+    //    the latency of the 3-deep HBM pipeline, profiles/r01_ncu_chain.md), so the slabs equalise the number of stages
+    //    per CTA rather than bytes: 10 job types x ~14.8 slabs = 147 CTAs on a whole GPU.
+    const int ctas = std::min(num_sms() - 1, kMaxWgradJobs);
+    WgradJobs jobs;
+    int nj = 0;
+    auto add_jobs = [&](int tg, int tx, int mblk, int nblk, float* dW, int ldw, int col0, int enc, int slabs, float* colsum) {
+      slabs = std::max(1, std::min(slabs, ntiles));
+      for (int sl = 0; sl < slabs; ++sl, ++nj) {
+        if (nj >= kMaxWgradJobs) continue;   // counted, rejected below
+        WgradJob& j = jobs.j[nj];
+        j.t_g = tg; j.t_x = tx; j.mblk = mblk; j.nblk = nblk;
+        j.tile_begin = (int)((long long)ntiles * sl / slabs);
+        j.tile_end = (int)((long long)ntiles * (sl + 1) / slabs);
+        j.dW = dW; j.ldw = ldw; j.col0 = col0; j.enc_cols = enc; j.colsum = colsum;
+        j.passes = wg_passes;
+      }
     };
-    // (bias gradients = column sums of the gradient images are produced inside the weight-gradient kernel)
-    add_red(T_H0 + 6, 4, 1, c.g_raw, 1, grad->trunk_w[7], kW, grad->trunk_b[7]);        // density row of trunk 7
-    add_red(T_HID, 2, 3, c.g_pre, 4, grad->head_w[1], kHW, grad->head_b[1]);             // 128 -> 3 colour layer
+    int slabs[10];      // 8 wide job types, then the two encoder-block types
+    const int s_lo = std::max(1, ctas / 10), extra = std::max(0, std::min(8, ctas - 10 * s_lo));
+    for (int i = 0; i < 10; ++i) slabs[i] = s_lo + (i < extra ? 1 : 0);
+    add_jobs(T_GHID, T_FEAT, 2, 4, grad->head_w[0], kW + kEv, 0, 0, slabs[7], grad->head_b[0]);     // head 0, feature part
+    add_jobs(T_G7F, T_H0 + 6, 4, 4, grad->trunk_w[7] + kW, kW, 0, 0, slabs[0], grad->trunk_b[7] + 1);  // trunk 7 rows 1..256
+    for (int l = 6; l >= 1; --l)
+      add_jobs(t_g(l), T_H0 + (l - 1), 4, 4, grad->trunk_w[l], l == 4 ? kW + 63 : kW, 0, 0, slabs[7 - l], grad->trunk_b[l]);
+    add_jobs(t_g(4), T_ENC, 4, 1, grad->trunk_w[4], kW + 63, kW, 1, slabs[8], nullptr);             // skip part of layer 4
+    add_jobs(t_g(0), T_ENC, 4, 1, grad->trunk_w[0], 63, 0, 1, slabs[9], grad->trunk_b[0]);          // layer 0 (+ its bias)
+    SPARF_REQUIRE(nj <= kMaxWgradJobs, "tc_mlp_backward: %d weight-gradient jobs exceed the table of %d", nj, kMaxWgradJobs);
+    tc_mlp_wgrad_kernel<<<nj, 192, kWgSmem + 1024, st>>>(jobs, img);
+    SPARF_CHECK_LAUNCH("tc_mlp_wgrad_kernel");
+
+    // 4. CUDA-core leftovers: density row, 128->3 head, view-direction columns (bias gradients = column sums of the
+    //    gradient images are produced inside the weight-gradient kernel)
+    const int parts = (tape && wg_passes == 1) ? 1 : 2;     // forward images of a TC_3X_W1 tape hold their hi halves only
+    const ReduceJob density{T_H0 + 6, 4, 1, c.g_raw, 1, grad->trunk_w[7], kW, grad->trunk_b[7], parts};   // density row of trunk 7
+    const ReduceJob colour{T_HID, 2, 3, c.g_pre, 4, grad->head_w[1], kHW, grad->head_b[1], parts};         // 128 -> 3 colour layer
     const int tpb = 4;
-    // one launch per job shape (blockIdx.y = job index is passed through the first table entry of each launch)
-    ReduceJobs one;
-    one.j[0] = rj[0];
-    image_reduce_kernel<1><<<dim3(ceil_div(ntiles, tpb), 1), 256, 0, sd>>>(one, img, Mc, ntiles, tpb);
+    image_reduce_kernel<1><<<ceil_div(ntiles, tpb), 256, 0, sd>>>(density, img, Mc, ntiles, tpb);
     SPARF_CHECK_LAUNCH("image_reduce_kernel<1>");
-    one.j[0] = rj[1];
-    image_reduce_kernel<3><<<dim3(ceil_div(ntiles, tpb), 1), 256, 0, sd2>>>(one, img, Mc, ntiles, tpb);
+    image_reduce_kernel<3><<<ceil_div(ntiles, tpb), 256, 0, sd2>>>(colour, img, Mc, ntiles, tpb);
     SPARF_CHECK_LAUNCH("image_reduce_kernel<3>");
     ray_sum_ghid_kernel<<<nr, 128, 0, sd2>>>(img, nr, S, c.rayS);
     SPARF_CHECK_LAUNCH("ray_sum_ghid_kernel");
@@ -2556,15 +2271,14 @@ static int tc_mlp_backward_impl(const SparfMLP* mlp, int engine, int R, int S, c
         SPARF_CHECK_LAUNCH("direnc_bwd_kernel");
       }
     }
-    if (side) {   // join: later work on the caller's stream (next chunk, optimiser, ...) sees every gradient
-      SPARF_CHECK_CUDA(cudaEventRecord(side->join, side->stream));
-      SPARF_CHECK_CUDA(cudaStreamWaitEvent(st, side->join, 0));
-      if (sd2 != sd) {
-        SPARF_CHECK_CUDA(cudaEventRecord(side->join2, sd2));
-        SPARF_CHECK_CUDA(cudaStreamWaitEvent(st, side->join2, 0));
-        SPARF_CHECK_CUDA(cudaEventRecord(side->join3, sd3));
-        SPARF_CHECK_CUDA(cudaStreamWaitEvent(st, side->join3, 0));
-      }
+    // join: later work on the caller's stream (next chunk, optimiser, ...) sees every gradient
+    SPARF_CHECK_CUDA(cudaEventRecord(side->join, side->stream));
+    SPARF_CHECK_CUDA(cudaStreamWaitEvent(st, side->join, 0));
+    if (sd2 != sd) {
+      SPARF_CHECK_CUDA(cudaEventRecord(side->join2, sd2));
+      SPARF_CHECK_CUDA(cudaStreamWaitEvent(st, side->join2, 0));
+      SPARF_CHECK_CUDA(cudaEventRecord(side->join3, sd3));
+      SPARF_CHECK_CUDA(cudaStreamWaitEvent(st, side->join3, 0));
     }
   }
   return SPARF_OK;

@@ -18,12 +18,9 @@ def test_cold_l2_repetitions_are_reproducible(monkeypatch, capsys):
     assert "stress ok: 40 repetitions" in capsys.readouterr().out
 
 
-# every kernel variant that stays selectable (the knobs are read once per process, hence subprocesses), plus a batch
-# larger than one backward chunk (chunked tape walk with accumulating gradients)
+# the recompute backward (its bf16 forward runs the shared-memory-operand chain kernel), plus a batch larger than one
+# backward chunk (chunked tape walk with accumulating gradients); subprocesses, one per variant
 VARIANTS = [
-    ("shared-memory-operand chain kernels", {"SPARF_TC_TMEMA": "0"}, ["25"]),
-    ("backward pipelined in 3 sub-chunks", {"SPARF_TC_BWD_SPLIT": "3"}, ["25"]),
-    ("no side stream", {"SPARF_TC_OVERLAP": "0"}, ["25"]),
     ("recompute backward (no tape)", {"STRESS_TAPE": "0"}, ["25"]),
     ("two backward chunks", {}, ["15", "1100", "128"]),
 ]

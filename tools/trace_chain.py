@@ -1,8 +1,9 @@
 #!/usr/bin/env python
 """Wait-time breakdown of the warp roles of the tcgen05 chain kernels.
 
-Needs a library built with SPARF_NVCC_DEFINES=-DSPARF_TC_TRACE (the kernels then accumulate, per role, the clocks spent
-in each mbarrier wait and print the mean over CTAs to stderr after every launch).  Debug tool, not part of the product.
+Needs the tracing library, built by `python -m sparf_b200.build --trace` and loaded with
+SPARF_B200_LIB=sparf_b200/lib/libsparf_b200_trace.so (the kernels then accumulate, per role, the clocks spent in each
+mbarrier wait and print the mean over CTAs to stderr after every launch).  Debug tool, not part of the product.
 """
 import os
 import sys
